@@ -41,6 +41,8 @@ DEFAULTS = dict(workload="spp-608", batch=64, kind="B", conf=0.3, nms=0.5)
 # images per CPU measurement: the whole batch where the reference gets through it in seconds (same config as the GPU
 # arm), a bounded sample of it otherwise (SURVEY 8d: about 10-30 s of CPU work per leg)
 WARM_SECONDS = 0.04          # minimum duration of the untimed warm-up (see Case.timed)
+DEFAULT_STEPS = 2000
+DUMP_LIMIT_BYTES = 64 << 20  # --dump-outputs: all files together
 CPU_SAMPLE_BATCH = {"spp-608": 64, "spp-1024": 8, "tiny-416": 256}
 # the other BASELINE.json configs, measured in the same run (bounded): (label, workload, batch/GPU, kind, conf, nms)
 EXTRA_CONFIGS = [
@@ -53,7 +55,8 @@ EXTRA_CONFIGS = [
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=None,
+                    help=f"timed steps (default {DEFAULT_STEPS}; --impl reference: as many as --ref-budget-s allows)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=DEFAULTS["workload"])
@@ -76,8 +79,14 @@ def parse_args():
     ap.add_argument("--config-steps", type=int, default=30)
     ap.add_argument("--cpu-runs", type=int, default=5)
     ap.add_argument("--cpu-kind", default="reference", choices=["reference", "port"])
-    ap.add_argument("--ref-budget-s", type=float, default=150.0, help="--impl reference: wall-clock budget of the timed steps")
-    return ap.parse_args()
+    ap.add_argument("--ref-budget-s", type=float, default=150.0,
+                    help="--impl reference without --steps: wall-clock budget of the timed steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def default_batch(workload):
@@ -153,7 +162,8 @@ def physical_gpu_index(local_index: int) -> int:
 def cpu_run(kind, workload, batch, synth_kind, conf, nms, runs, warm=1, budget_s=None):
     """Times the reference path on the host cores: ``kind == "reference"`` runs the UNMODIFIED reference functions
     (YOLOLayer.forward per scale + torch.cat + non_max_suppression, loaded by path from oracle/_ref or the reference
-    checkout); ``"port"`` runs the oracle restatement.  Returns (images/s of the median run, per-run seconds, kind used)."""
+    checkout); ``"port"`` runs the oracle restatement.  Returns (images/s of the median run, per-run seconds, kind used,
+    the detections of the last run)."""
     from pytorch_yolo_b200 import synth
     w = synth.WORKLOADS[workload]
     heads = synth.synth_heads(workload, batch, synth_kind, seed=1234)
@@ -183,13 +193,13 @@ def cpu_run(kind, workload, batch, synth_kind, conf, nms, runs, warm=1, budget_s
     with torch.no_grad():
         for i in range(warm + runs):
             t0 = time.perf_counter()
-            fn()
+            dets = fn()
             dt = time.perf_counter() - t0
             if i >= warm:
                 times.append(dt)
             if budget_s is not None and times and time.perf_counter() - t_start + dt > budget_s:
                 break
-    return batch / statistics.median(times), times, kind
+    return batch / statistics.median(times), times, kind, dets
 
 
 def cpu_tiny_model_run(runs=10):
@@ -232,10 +242,13 @@ def run_reference(args):
     torch.set_num_threads(cores)
     full_b = args.batch
     sample_b = min(full_b, CPU_SAMPLE_BATCH.get(args.workload, 8))
-    steps = max(1, args.steps)
     warm = max(1, min(args.warmup, 2))
-    ips, times, kind = cpu_run(args.cpu_kind, args.workload, sample_b, args.kind, args.conf, args.nms, runs=steps, warm=warm,
-                               budget_s=args.ref_budget_s)
+    ips, times, kind, dets = cpu_run(args.cpu_kind, args.workload, sample_b, args.kind, args.conf, args.nms,
+                                     runs=args.steps or DEFAULT_STEPS, warm=warm,
+                                     budget_s=args.ref_budget_s if args.steps is None else None)
+    if args.dump_outputs:
+        from pytorch_yolo_b200 import synth
+        dump_outputs(args.dump_outputs, dets, None, synth.anchors_per_image(args.workload))
     sample = (f"{args.workload} SYNTH-{args.kind} {sample_b} of {full_b} images per step, conf {args.conf} nms {args.nms}, "
               f"{len(times)} timed steps (median), torch threads {torch.get_num_threads()}")
     line = {
@@ -258,6 +271,38 @@ def workload_config(args, batch):
             "l2": "inputs exceed L2 (no flush needed)" if synth.head_bytes_per_image(args.workload) * batch > 126e6
                   else "inputs rotate through >L2 worth of buffers",
             "sharding": "images across GPUs, kept rows to rank 0 by NVLink peer stores"}
+
+
+def dump_outputs(path, dets, rows, cap):
+    """--dump-outputs: what the caller of the timed path received from its last step, as .npy files in `path`, so that
+    two builds can be compared output for output (the inputs depend only on the arguments).
+      detections.npy      float32 (n, 7)  kept rows (x1, y1, x2, y2, obj, cls_conf, cls) of the dumped images, in order
+      kept_per_image.npy  float64         number of those rows per dumped image
+      image_index.npy     float64         which images of the batch were dumped
+      anchor_rows.npy     float64 (n,)    anchor row each kept row came from (GPU arm only)
+    `dets` / `rows`: per image an (n, 7) / (n,) tensor or None; `cap`: most rows one image can keep.  All images are
+    dumped when their largest possible result fits DUMP_LIMIT_BYTES, else a fixed seeded sample of them, which depends
+    only on the batch size and `cap`."""
+    import numpy as np
+    per_image = cap * (7 * 4 + (8 if rows is not None else 0)) + 16
+    take = min(len(dets), (DUMP_LIMIT_BYTES - 1024) // per_image)       # 1024: the .npy headers
+    if take == len(dets):
+        index = torch.arange(len(dets))
+    else:
+        index = torch.randperm(len(dets), generator=torch.Generator().manual_seed(0))[:take].sort().values
+    index = index.tolist()
+    kept = [0 if dets[i] is None else len(dets[i]) for i in index]
+    arrays = {
+        "detections": torch.cat([dets[i].cpu() for i in index if dets[i] is not None] + [torch.empty(0, 7)]).numpy(),
+        "kept_per_image": np.array(kept, dtype=np.float64),
+        "image_index": np.array(index, dtype=np.float64),
+    }
+    if rows is not None:
+        arrays["anchor_rows"] = torch.cat([rows[i].cpu().double() for i in index if rows[i] is not None]
+                                          + [torch.empty(0, dtype=torch.float64)]).numpy()
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------- one workload on the GPU(s)
@@ -386,6 +431,14 @@ class Case:
             by_rank = [float(x.item()) / steps for x in every]
             elapsed_ms = max(float(x.item()) for x in every)          # the job is as slow as its slowest rank
         return elapsed_ms, by_rank, cand
+
+    def last_result(self, steps):
+        """What the caller got from the last of `steps` timed steps: (per-image (n, 7) detections, anchor rows), None
+        for an image without any.  N > 1: the gathered global batch on rank 0, None on the other ranks."""
+        if self.det is not None:
+            return self.det.gather(self.det.pipe._next - 1, return_rows=True)
+        p = self.pipes[(steps - 1) % self.n_sets]          # run_steps' choice for step steps - 1
+        return p.collect(p._next - 1, return_rows=True)
 
     def kernel_roofline(self, cand_total, peak, peak_src, reps):
         """The dominant kernel (decode_compact) timed alone with CUDA events on its stream."""
@@ -701,6 +754,7 @@ def main():
         args.no_cpu_baseline = args.no_e2e = args.no_head_fusion = args.no_configs = args.no_drop_in = True
     if args.impl == "reference":
         return run_reference(args)
+    args.steps = args.steps or DEFAULT_STEPS
 
     import torch.distributed as dist
     from pytorch_yolo_b200 import hostmem, ops
@@ -724,6 +778,11 @@ def main():
     sampler = ClockSampler(physical_gpu_index(local_rank))
     elapsed_ms, by_rank, cand_total = case.timed(args.steps, args.warmup, sampler)
     clocks = sampler.finish()
+    if args.dump_outputs:
+        # before anything else runs on the lanes' buffers
+        res = case.last_result(args.steps)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, *res, case.lane0.buf.out_cap)
     value = B * world * args.steps / (elapsed_ms * 1e-3)
     roofline = case.kernel_roofline(cand_total, peak, peak_src, reps=max(20, min(args.steps, 200)))
     lane0 = case.lane0
@@ -783,7 +842,7 @@ def main():
         cores = os.cpu_count() or 1
         torch.set_num_threads(cores)
         sb = min(B, CPU_SAMPLE_BATCH.get(args.workload, 8))
-        ips, times, kind = cpu_run(args.cpu_kind, args.workload, sb, args.kind, args.conf, args.nms, runs=args.cpu_runs)
+        ips, times, kind, _ = cpu_run(args.cpu_kind, args.workload, sb, args.kind, args.conf, args.nms, runs=args.cpu_runs)
         line["cpu_baseline"] = {"value": ips, "unit": UNIT, "cores": cores, "kind": kind,
                                 "sample": f"{args.workload} SYNTH-{args.kind} batch {sb}, {len(times)} runs (median), "
                                           f"{sum(times):.1f} s of CPU work, torch threads {torch.get_num_threads()}: "

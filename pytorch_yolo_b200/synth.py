@@ -97,16 +97,20 @@ def _plant_objects(heads: Sequence[torch.Tensor], w: dict, gen: torch.Generator,
         gy = torch.clamp((cy / s).floor().long(), 0, g - 1)
         fx = torch.clamp(cx / s - gx, 0.05, 0.95)
         fy = torch.clamp(cy / s - gy, 0.05, 0.95)
+        # objects of one image in one cell: the last one is planted, as by one write after the other (an indexed
+        # assignment with repeated indices leaves the winner to the thread schedule: inputs would differ run to run)
+        cell = gy * g + gx
+        keep = ~(cell.unsqueeze(2) == cell.unsqueeze(1)).triu(1).any(2)
+        kb, ky, kx = bi[keep], gy[keep], gx[keep]
         for a, (aw, ah) in enumerate(anchors):
-            h[bi, a, 0, gy, gx] = torch.logit(fx) + 0.3 * nrm(batch, n_obj)
-            h[bi, a, 1, gy, gx] = torch.logit(fy) + 0.3 * nrm(batch, n_obj)
-            h[bi, a, 2, gy, gx] = torch.log(bw / aw) + 0.1 * nrm(batch, n_obj)
-            h[bi, a, 3, gy, gx] = torch.log(bh / ah) + 0.1 * nrm(batch, n_obj)
-            h[bi, a, 4, gy, gx] = 2.0 + 1.5 * nrm(batch, n_obj)
+            h[kb, a, 0, ky, kx] = (torch.logit(fx) + 0.3 * nrm(batch, n_obj))[keep]
+            h[kb, a, 1, ky, kx] = (torch.logit(fy) + 0.3 * nrm(batch, n_obj))[keep]
+            h[kb, a, 2, ky, kx] = (torch.log(bw / aw) + 0.1 * nrm(batch, n_obj))[keep]
+            h[kb, a, 3, ky, kx] = (torch.log(bh / ah) + 0.1 * nrm(batch, n_obj))[keep]
+            h[kb, a, 4, ky, kx] = (2.0 + 1.5 * nrm(batch, n_obj))[keep]
             logits = -5.0 + nrm(batch, n_obj, nc)
             logits.scatter_(2, cls.unsqueeze(2), 4.0 + nrm(batch, n_obj, 1))
-            h[bi.unsqueeze(2), a, 5 + torch.arange(nc, device=dev).view(1, 1, nc),
-              gy.unsqueeze(2), gx.unsqueeze(2)] = logits
+            h[kb.unsqueeze(1), a, 5 + torch.arange(nc, device=dev).view(1, nc), ky.unsqueeze(1), kx.unsqueeze(1)] = logits[keep]
 
 
 def synth_prediction(batch: int, n_rows: int, nc: int = 80, seed: int = 0, img: float = 608.0,

@@ -1,6 +1,6 @@
 """The evaluation loop (SURVEY.md section 8f row 2) against records the LIVE reference produced.
 
-``tests/golden/eval_loop.npz`` holds the ``{path: [records]}`` dicts of the inner loop of the reference's ``test_model``
+``tests/golden/eval_loop.npz`` (with ``eval_loop_a1.npz``) holds the ``{path: [records]}`` dicts of the inner loop of the reference's ``test_model``
 (utils/utils.py:374-379; made by tests/golden/make_golden_eval.py).  CPU: the oracle's restatement of that loop reproduces
 them exactly.  GPU: (1) fed the reference's decoded tensor, the drop-in ``non_max_suppression`` + ``dict_from_results``
 give the same records -- scores and classes bit-exact, pixel coordinates equal except where a MERGE box (rtol 1e-5, see
@@ -23,7 +23,7 @@ SPP_SMALL = synth.WORKLOADS["mini-96"]
 
 
 def _golden():
-    g = load_golden("eval_loop")
+    g = {**load_golden("eval_loop"), **load_golden("eval_loop_a1")}
     tiny = load_golden("tiny416_randinit")
     model_a = dict(anchors=SPP_SMALL["anchors"], nc=SPP_SMALL["nc"], cur_shape=(96, 96), batches=[])
     for bi in range(2):
