@@ -469,6 +469,13 @@ def test_head_detector_fp32x3_matches_oracle_detections():
     img = int(round(specs[0].stride * max(specs[0].ny, specs[0].nx)))
     pred = yolo_oracle.decode_heads(hts, anchors, nc, img)
     want, want_rows = yolo_oracle.non_max_suppression_indexed(pred, conf, nms)
+    assert assert_fp32x3_detections_match_oracle(got, got_rows, want, want_rows) > 50
+
+
+def assert_fp32x3_detections_match_oracle(got, got_rows, want, want_rows, score_rtol=3e-5):
+    """The three-pass mode's detections against the oracle's on fp32 head tensors: kept anchor rows as sets up to one in
+    200, classes equal, scores within ``score_rtol`` relative, boxes within 1e-5 (1e-3 in an image with a one-sided
+    detection).  Returns the number of detections the oracle kept."""
     n_total = 0
     for g, gr, o, orow in zip(got, got_rows, want, want_rows):
         gset, oset = set(gr.cpu().tolist()), set(orow.tolist())
@@ -480,12 +487,13 @@ def test_head_detector_fp32x3_matches_oracle_detections():
         gsel = g.cpu()[[gi[r] for r in common]]
         osel = o[[oi[r] for r in common]]
         assert torch.equal(gsel[:, 6], osel[:, 6])                                   # class
-        # score, class confidence: the two fp32 convolutions sum c_in products in different orders, so a logit t differs by
-        # ~1e-6 * sum |w||x| (~1e-5 absolute here), which moves sigmoid(t) by (1 - sigmoid(t)) * dt relative: 3e-5 covers
-        # the accumulation order, 1e-5 is the bar on identical head tensors (test_gpu_parity.py)
-        torch.testing.assert_close(gsel[:, 4:6], osel[:, 4:6], rtol=3e-5, atol=1e-7)
+        # score, class confidence: the kernel's logits t are within ~2e-6 * sum |w||x| of fp64 (the tensor core's fp32
+        # accumulation over three passes; the oracle's CPU convolution is closer), which moves sigmoid(t) by
+        # (1 - sigmoid(t)) * dt relative: 3e-5 covers that for the spp_like heads (c_in <= 256); 1e-5 is the bar on
+        # identical head tensors (test_gpu_parity.py)
+        torch.testing.assert_close(gsel[:, 4:6], osel[:, 4:6], rtol=score_rtol, atol=1e-7)
         # boxes: a MERGE box averages its cluster, so a member that differs between the two sides moves it; compare the
         # rows whose clusters cannot have changed (no one-sided detection in the image) strictly, the others loosely
         tol = 1e-5 if gset == oset else 1e-3
         torch.testing.assert_close(gsel[:, :4], osel[:, :4], rtol=tol, atol=tol * 600)
-    assert n_total > 50
+    return n_total
