@@ -88,9 +88,11 @@ int yolo_b200_decode_compact(const yolo_b200_scale* scales_host, int n_scales, i
                              yolo_b200_box* cand_box, yolo_b200_meta* cand_meta, int cap_per_img,
                              int32_t* count, int32_t* overflow, yolo_b200_stream_t stream);
 
-/* Same call with an explicit kernel variant: 0 = automatic, 1 = LDG kernel (many small CTAs, 128-bit
- * coalesced loads), 2 = TMA kernel (persistent CTAs, ring of 1-D cp.async.bulk copies), 3 = the same kernel fed by one
- * 2-D tensor-map copy per tile (needs 5+n_classes <= 256).  All produce identical candidates. */
+/* Same call with an explicit kernel variant: 0 = automatic (= 1), 1 = gated LDG kernel (many small CTAs, 128-bit
+ * coalesced loads; reads the objectness plane first and the box and class planes only around positions whose objectness
+ * can pass conf_thres), 2 = TMA kernel (persistent CTAs, ring of 1-D cp.async.bulk copies), 3 = the same kernel fed by one
+ * 2-D tensor-map copy per tile (needs 5+n_classes <= 256), 4 = dense LDG kernel (variant 1 without the gate: reads every
+ * plane).  Variants 2 to 4 read the whole head tensor.  All produce identical candidates. */
 int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales_host, int n_scales, int batch, int n_classes,
                                 int rows_per_img, float conf_thres, float min_wh,
                                 yolo_b200_box* cand_box, yolo_b200_meta* cand_meta, int cap_per_img,

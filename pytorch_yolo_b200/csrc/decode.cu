@@ -7,7 +7,9 @@
 //   compact_from_dense_kernel  the filter/compaction half of non_max_suppression on an already decoded
 //                              tensor (reference utils/utils.py:210-234), fed by TMA bulk copies
 //
-// All three are HBM-bound streaming kernels: each input byte is read exactly once.
+// All three are HBM-bound streaming kernels that read each input byte at most once.  decode_compact_kernel reads the
+// objectness plane whole and the box and class planes only around positions whose objectness can pass the confidence
+// threshold; decode_compact_dense_kernel (selectable) and the other kernels read every byte once.
 #include <cuda.h>          // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 
 #include "common.cuh"
@@ -140,35 +142,36 @@ __device__ __forceinline__ void finish_anchor(const DecodeParams& P, const Scale
     }
 }
 
-template <int VEC, int kDcUnroll>
-__device__ __forceinline__ void decode_compact_body(const DecodeParams& P, const ScaleDev& S, int block_local) {
-    const int nc = P.nc;
-    const int no = nc + 5;
-    const int plane = S.plane;
-    const int pv_per_slab = plane / VEC;
+// One work unit of the LDG kernels: VEC consecutive positions of one (image, anchor) slab.  Units past the end are
+// clamped onto the last one (a valid address) and marked inactive, so that the lane still takes part in the collectives.
+struct DcUnit {
+    const float* base;   // channel 0 of the unit's first position
+    int img, a, pos0;
+    bool active;
+};
 
-    int unit = block_local * kDcThreads + (int)threadIdx.x;
-    const bool active = unit < S.n_units;
-    if (!active) unit = S.n_units - 1;            // keep the lane alive for the warp collectives
+template <int VEC>
+__device__ __forceinline__ DcUnit dc_unit(const ScaleDev& S, int no, int unit) {
+    DcUnit u;
+    u.active = unit < S.n_units;
+    if (!u.active) unit = S.n_units - 1;
+    const int pv_per_slab = S.plane / VEC;
     const int slab = unit / pv_per_slab;
     const int pv = unit - slab * pv_per_slab;
-    const int img = slab / S.na;
-    const int a = slab - img * S.na;
-    const int pos0 = pv * VEC;
-    const float* base = S.head + (size_t)slab * no * plane + pos0;
+    u.img = slab / S.na;
+    u.a = slab - u.img * S.na;
+    u.pos0 = pv * VEC;
+    u.base = S.head + (size_t)slab * no * S.plane + u.pos0;
+    return u;
+}
 
-    // box + objectness planes
-    float t[5][VEC];
-#pragma unroll
-    for (int c = 0; c < 5; ++c) load_vec<VEC>(t[c], base + (size_t)c * plane);
-
-    // running (max, second max, first arg-max) over the class planes; max propagates NaN
-    float m[VEC], m2[VEC];
-    int idx[VEC];
+// Running (max, second max, first arg-max) over the class planes at cbase, kDcUnroll planes in flight per batch; the max
+// propagates NaN.
+template <int VEC, int kDcUnroll>
+__device__ __forceinline__ void scan_classes(const float* cbase, int plane, int nc, float (&m)[VEC], float (&m2)[VEC],
+                                             int (&idx)[VEC]) {
 #pragma unroll
     for (int j = 0; j < VEC; ++j) { m[j] = __int_as_float(0xff800000); m2[j] = m[j]; idx[j] = 0; }
-
-    const float* cbase = base + (size_t)5 * plane;
     int c0 = 0;
     auto scan = [&](const float (&v)[kDcUnroll][VEC], int cfirst) {
 #pragma unroll
@@ -206,24 +209,102 @@ __device__ __forceinline__ void decode_compact_body(const DecodeParams& P, const
             }
         }
     }
+}
+
+// Dense: one unit per thread, every plane read.
+template <int VEC, int kDcUnroll>
+__device__ __forceinline__ void decode_compact_dense_body(const DecodeParams& P, const ScaleDev& S, int block_local) {
+    const int plane = S.plane;
+    const DcUnit u = dc_unit<VEC>(S, P.nc + 5, block_local * kDcThreads + (int)threadIdx.x);
+
+    // box + objectness planes
+    float t[5][VEC];
+#pragma unroll
+    for (int c = 0; c < 5; ++c) load_vec<VEC>(t[c], u.base + (size_t)c * plane);
+
+    float m[VEC], m2[VEC];
+    int idx[VEC];
+    const float* cbase = u.base + (size_t)5 * plane;
+    scan_classes<VEC, kDcUnroll>(cbase, plane, P.nc, m, m2, idx);
 
 #pragma unroll
     for (int j = 0; j < VEC; ++j)
-        finish_anchor(P, S, active, img, a, pos0 + j, t[0][j], t[1][j], t[2][j], t[3][j], t[4][j],
+        finish_anchor(P, S, u.active, u.img, u.a, u.pos0 + j, t[0][j], t[1][j], t[2][j], t[3][j], t[4][j],
                       m[j], m2[j], idx[j], cbase + j, plane);
 }
 
+// Objectness gate.  finish_anchor's first test is fl(fl(so * sm) * kSlack) > conf with so = sigmoidf_rn(t4) and
+// sm = sigmoidf_rn(max class logit) (or 1 for one class).  sigmoidf_rn ends in rcp.approx(1 + e) with 1 + e >= 1, and
+// rcp.approx is within 1 ulp, so sm <= 1 + 2^-23; with the two roundings the left side is at most
+// so * 1.00003 * (1 + 2^-23) * (1 + 2^-24)^2 < so * 1.0000305 for so >= 0.  The gate computes fl(so * 1.0001), which is
+// >= so * 1.0001 * (1 - 2^-24) > so * 1.0000305: whenever the test can pass, the gate passes.  so is the very value
+// finish_anchor computes from the same t4.  NaN objectness gives so = NaN and a false gate, as the test is false there
+// too; -inf gives so = 0, which passes only if conf < 0, like the test.
+__device__ __forceinline__ bool obj_gate(float t4, float conf) {
+    return __fmul_rn(sigmoidf_rn(t4), 1.0001f) > conf;
+}
 
-__global__ void __launch_bounds__(kDcThreads, YB_DC_MINBLOCKS)
-decode_compact_kernel(const __grid_constant__ DecodeParams P) {
+// Gated: one unit per thread, as in the dense kernel, but the objectness plane is read first and the box and class
+// planes only for units with a position that passes obj_gate, so only the 32-byte sectors some passing anchor needs are
+// requested.  With every position passing, a thread issues the loads of the dense kernel, one round trip later.
+// (Variants that prefetch the objectness of a second or fourth unit per thread while scanning the current one were
+// slower on every configuration but conf 0.001: DESIGN.md section 6.)
+template <int VEC, int kDcUnroll>
+__device__ __forceinline__ void decode_compact_gated_body(const DecodeParams& P, const ScaleDev& S, int block_local) {
+    const int plane = S.plane;
+    const DcUnit u = dc_unit<VEC>(S, P.nc + 5, block_local * kDcThreads + (int)threadIdx.x);
+    float t[5][VEC];
+    load_vec<VEC>(t[4], u.base + (size_t)4 * plane);
+    bool gate[VEC];
+    bool any = false;
+#pragma unroll
+    for (int j = 0; j < VEC; ++j) {
+        gate[j] = u.active && obj_gate(t[4][j], P.conf);
+        any |= gate[j];
+    }
+    float m[VEC], m2[VEC];
+    int idx[VEC];
+    const float* cbase = u.base + (size_t)5 * plane;
+    if (any) {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) load_vec<VEC>(t[c], u.base + (size_t)c * plane);
+        scan_classes<VEC, kDcUnroll>(cbase, plane, P.nc, m, m2, idx);
+    } else {                                                   // finish_anchor reads none of these for a gated-off position
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) {
+            t[0][j] = t[1][j] = t[2][j] = t[3][j] = 0.0f;
+            m[j] = m2[j] = 0.0f;
+            idx[j] = 0;
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < VEC; ++j)
+        finish_anchor(P, S, gate[j], u.img, u.a, u.pos0 + j, t[0][j], t[1][j], t[2][j], t[3][j], t[4][j],
+                      m[j], m2[j], idx[j], cbase + j, plane);
+}
+
+__device__ __forceinline__ const ScaleDev& dc_scale(const DecodeParams& P) {
     int s = 0;
 #pragma unroll
     for (int k = 1; k < YOLO_B200_MAX_SCALES; ++k)
         if (k < P.n_scales && (int)blockIdx.x >= P.sc[k].first_block) s = k;
-    const ScaleDev& S = P.sc[s];
+    return P.sc[s];
+}
+
+__global__ void __launch_bounds__(kDcThreads, YB_DC_MINBLOCKS)
+decode_compact_kernel(const __grid_constant__ DecodeParams P) {
+    const ScaleDev& S = dc_scale(P);
     const int block_local = (int)blockIdx.x - S.first_block;
-    if (S.vec == 4) decode_compact_body<4, YB_DC_UNROLL>(P, S, block_local);
-    else            decode_compact_body<1, YB_DC_UNROLL1>(P, S, block_local);
+    if (S.vec == 4) decode_compact_gated_body<4, YB_DC_UNROLL>(P, S, block_local);
+    else            decode_compact_gated_body<1, YB_DC_UNROLL1>(P, S, block_local);
+}
+
+__global__ void __launch_bounds__(kDcThreads, YB_DC_MINBLOCKS)
+decode_compact_dense_kernel(const __grid_constant__ DecodeParams P) {
+    const ScaleDev& S = dc_scale(P);
+    const int block_local = (int)blockIdx.x - S.first_block;
+    if (S.vec == 4) decode_compact_dense_body<4, YB_DC_UNROLL>(P, S, block_local);
+    else            decode_compact_dense_body<1, YB_DC_UNROLL1>(P, S, block_local);
 }
 
 // ---- mbarrier / TMA bulk-copy helpers --------------------------------------------------------------
@@ -910,8 +991,9 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     if (!cand_box || !cand_meta || !count || !overflow) return YOLO_B200_E_NULL;
     const bool accumulate = variant >= 0 && (variant & YOLO_B200_VARIANT_ACCUMULATE) != 0;
     if (accumulate) variant &= ~YOLO_B200_VARIANT_ACCUMULATE;
-    if (cap_per_img < 1 || variant < 0 || variant > 3) return YOLO_B200_E_RANGE;
+    if (cap_per_img < 1 || variant < 0 || variant > 4) return YOLO_B200_E_RANGE;
     if ((((uintptr_t)cand_box) | ((uintptr_t)cand_meta)) & 15u) return YOLO_B200_E_ALIGN;
+    const bool gated = variant <= 1;
     DecodeParams P{};
     const int blocks = fill_params(P, scales, n_scales, batch, nc, rows_per_img, false, accumulate);
     if (blocks < 0) return blocks;
@@ -925,11 +1007,12 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int no = nc + 5;
     const int tp = tma_tile_positions(no);
-    // Measured on B200 (profiles/r01_c_decode_variants.txt): the LDG kernel streams at 5.8 TB/s, the 1-D bulk-copy
-    // ring at 3.1 TB/s (one cp.async.bulk per 1 KB channel row: TMA issue-bound), so "automatic" means LDG; the
-    // TMA variants stay selectable for comparison (2 = 1-D bulk copies, 3 = one 2-D tensor-map copy per tile).
-    const bool use_tma = tp > 0 && variant >= 2;
-    if (variant >= 2 && tp == 0) return YOLO_B200_E_RANGE;
+    // Measured on B200 (profiles/r01_c_decode_variants.txt): the dense LDG kernel streams at 5.8 TB/s, the 1-D bulk-copy
+    // ring at 3.1 TB/s (one cp.async.bulk per 1 KB channel row: TMA issue-bound), so "automatic" means LDG, and the gated
+    // LDG kernel reads box and class planes only where the objectness can pass (profiles/gated_decode_probe.txt).  The
+    // others stay selectable for comparison (2 = 1-D bulk copies, 3 = one 2-D tensor-map copy per tile, 4 = dense LDG).
+    const bool use_tma = variant == 2 || variant == 3;
+    if (use_tma && tp == 0) return YOLO_B200_E_RANGE;
     P.use_tmap = 0;
     if (use_tma) {
         const int rc = tile_table(P, n_scales, batch, no, tp, variant == 3);
@@ -943,8 +1026,10 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
             return (int)e;
         const int grid = (int)(tiles < sms ? tiles : sms);
         decode_compact_tma_kernel<<<grid, kTcThreads, smem, stream>>>(P);
-    } else {
+    } else if (gated) {
         decode_compact_kernel<<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
+    } else {
+        decode_compact_dense_kernel<<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
     }
     return (int)cudaGetLastError();
 }

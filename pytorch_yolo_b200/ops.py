@@ -168,14 +168,14 @@ def get_buffers(device, batch: int, cap: int, nc: int, max_per_class: int = MAX_
     return buf
 
 
-DECODE_VARIANTS = {"auto": 0, "ldg": 1, "tma": 2, "tma2d": 3}
+DECODE_VARIANTS = {"auto": 0, "ldg": 1, "tma": 2, "tma2d": 3, "ldg_dense": 4}
 
 
 def decode_compact(heads, specs, nc: int, conf_thres: float, buf: Buffers, min_wh: float = MIN_WH,
                    variant: str = "auto", row_offs: Optional[Sequence[int]] = None,
                    rows_per_img: Optional[int] = None, accumulate: bool = False) -> None:
     """Fused decode + filter + compaction into ``buf`` (no (B, N, 5+nc) tensor is materialised).
-    ``variant``: "auto" | "ldg" | "tma" | "tma2d" (identical results; see include/yolo_b200.h).
+    ``variant``: "auto" | "ldg" | "tma" | "tma2d" | "ldg_dense" (identical results; see include/yolo_b200.h).
     ``row_offs`` / ``rows_per_img`` / ``accumulate``: decode only some scales of a model and append to the candidates
     already in ``buf`` (the other scales went through :func:`head_decode_compact`)."""
     lib = _lib.load()
