@@ -37,9 +37,12 @@ __device__ __forceinline__ float fmax_nan(float a, float b) {
 
 // ---- the decode arithmetic (reference models/yolo_layer.py:91-94, SURVEY.md App. A) ---------------
 // sigma(x) = 1 / (1 + exp(-x)) on the SFU: one FMUL, MUFU.EX2, one FADD, MUFU.RCP (explicit PTX, so every kernel
-// evaluates the identical sequence).  ex2.approx is accurate to 2^-22 and rcp.approx to 1 ulp; the scaling of
-// the argument adds |x| * 2^-24, so the relative error is <= 4e-7 + 6e-8 * |x| (<= 1e-6 for |x| <= 10, 6e-6 at
-// the fp32 overflow edge |x| = 88) against the 1e-5 the parity criterion allows.  An 85-channel row costs
+// evaluates the identical sequence).  ex2.approx is accurate to 2^-22, fl(1 + e) adds 2^-24 and rcp.approx 1 ulp
+// (2^-23): 4.2e-7.  The argument fl(x * fl(-log2 e)) carries the rounding of the product (2^-24) and of log2 e to fp32
+// (1.34e-8), which the exponential turns into |x| * 7.3e-8.  So the relative error is <= 4.2e-7 + 7.3e-8 * |x|
+// (<= 1.2e-6 for |x| <= 10, < 6.9e-6 up to the fp32 overflow edge |x| = 88) against the 1e-5 the parity criterion
+// allows; tests/test_gpu_decode_numerics.py holds every fp32 with 2^-8 <= |x| <= 128 to it, and
+// profiles/sigmoid_error_probe.txt has the measured worst case per binade.  An 85-channel row costs
 // 170 MUFU operations, which keeps the dense decode kernel HBM-bound instead of issue-bound.  The .ftz forms are
 // single instructions; they only differ for results below 1.2e-38 (logits under -87.3), which become 0.
 __device__ __forceinline__ float sigmoidf_rn(float x) {

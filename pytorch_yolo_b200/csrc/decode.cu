@@ -99,8 +99,9 @@ __device__ __forceinline__ void finish_anchor(const DecodeParams& P, const Scale
     const int nc = P.nc;
     const float stride = S.stride;
     const float conf = P.conf;
-    // more than twice the worst-case relative error of one sigmoid evaluation (6e-6 at |x| = 88, see common.cuh):
-    // if sigma(second largest logit) is further than this below sigma(largest), no other class can reach the max
+    // more than twice the worst-case relative error eps of one sigmoid evaluation (eps <= 4.2e-7 + 7.3e-8 * |x|, < 6.9e-6
+    // for |x| <= 88, see common.cuh): if sigma(second largest logit) is further than this below sigma(largest), no other
+    // class can reach the max.  That needs kSlack * (1 - 2^-24) >= (1 + eps) / (1 - eps): 1.00003 against 1.0000138
     const float kSlack = 1.00003f;
     bool emit = false;
     yolo_b200_box box = {0.f, 0.f, 0.f, 0.f};
