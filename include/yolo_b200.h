@@ -45,7 +45,9 @@ typedef struct CUstream_st* yolo_b200_stream_t;
 /* One detection scale = one YOLOLayer (models/yolo_layer.py:25-111).
  * Constants are what YOLOLayer.create_grids computes (yolo_layer.py:101-111). */
 typedef struct {
-    const float* head;      /* (B, na*(5+nc), ny, nx) fp32 NCHW contiguous: the tensor YOLOLayer.forward receives */
+    const float* head;      /* (B, na*(5+nc), ny, nx) fp32 NCHW contiguous: the tensor YOLOLayer.forward receives.
+                               yolo_b200_decode_compact_ex with YOLO_B200_VARIANT_F16 / _BF16 reads it as fp16 / bf16
+                               elements instead (2-byte aligned; 8-byte aligned planes take 8-byte loads) */
     int32_t ny, nx;         /* grid size (p.shape[-2], p.shape[-1]) */
     int32_t na;             /* anchors of this layer (len(anchors)) */
     int32_t row_off;        /* first row of this scale inside one image of the concatenated prediction
@@ -101,6 +103,13 @@ int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales_host, int n_scales
 /* OR-ed into `variant`: do not zero count / overflow first -- the candidates are appended to what earlier calls on the
  * same buffers produced (used when some scales of a model go through yolo_b200_head_decode_compact). */
 #define YOLO_B200_VARIANT_ACCUMULATE 0x100
+/* OR-ed into `variant` of yolo_b200_decode_compact_ex: every scale.head of the call holds fp16 (F16) or bf16 (BF16) elements.
+ * Each value is converted to fp32 as it is loaded, exactly, so the candidates are bit-identical to those of the same call on
+ * the fp32 upcast of the heads (this decodes in fp32; the reference run on 16-bit tensors rounds every op to 16 bits).
+ * Variants 0, 1 and 4 take them; with variant 2 or 3 the call returns YOLO_B200_E_UNSUPPORTED, with both bits
+ * YOLO_B200_E_RANGE, before anything is enqueued.  The other entry points read fp32 only. */
+#define YOLO_B200_VARIANT_F16 0x200
+#define YOLO_B200_VARIANT_BF16 0x400
 
 /* Same candidates, from an already decoded prediction (the tensor model.forward returned):
  * utils.py:210-234.  With write_back_score != 0 the product obj*max_cls is stored into

@@ -20,32 +20,33 @@ from pytorch_yolo_b200 import ops, synth  # noqa: E402
 
 CONFIGS = [("cfg2 spp-608 b64 conf 0.3", "spp-608", 64, 0.3), ("cfg3 tiny-416 b1024 conf 0.3", "tiny-416", 1024, 0.3),
            ("cfg4 spp-608 b64 conf 0.001", "spp-608", 64, 0.001), ("cfg5 spp-1024 b256 conf 0.3", "spp-1024", 256, 0.3)]
-POSITIONS_PER_UNIT = 4      # positions per unit when the plane is a multiple of 4 floats, else 1
+POSITIONS_PER_UNIT = 4      # positions per unit when the plane is a multiple of 4 elements, else 1
 
 
-def touched_bytes(heads, specs, nc, conf, gran):
+def touched_bytes(heads, specs, nc, conf, gran, esize=4):
     """Bytes in `gran`-byte granules the gated kernel requests: the whole objectness plane, and in each other plane the
-    granules holding a unit (4 or 1 positions) with a position that passes the gate.  Planes are counted one by one."""
+    granules holding a unit (4 or 1 positions) with a position that passes the gate.  Planes are counted one by one.
+    ``esize``: bytes per head element (4 for fp32 heads, 2 for fp16 / bf16 heads)."""
     no = nc + 5
     total = 0
     for h, s in zip(heads, specs):
         plane = s.ny * s.nx
         vec = POSITIONS_PER_UNIT if plane % 4 == 0 else 1
         v = h.view(-1, no, plane)                                          # slabs x channels x positions
-        so = torch.sigmoid(v[:, 4])
+        so = torch.sigmoid(v[:, 4].float())
         gate = (so * 1.0001) > conf
         unit = gate.view(v.shape[0], plane // vec, vec).any(-1)
         loaded = unit.repeat_interleave(vec, dim=1)                         # slabs x positions
         slabs = v.shape[0]
-        pos4 = torch.arange(plane, device=h.device) * 4
-        total += slabs * ((plane * 4 + gran - 1) // gran) * gran          # objectness plane (upper bound by one granule)
-        # plane c of slab s starts at byte ((s*no + c)*plane*4); its phase within a granule is one of gran/4 values
-        n_gran = (gran + plane * 4 + gran - 1) // gran
+        pos_b = torch.arange(plane, device=h.device) * esize
+        total += slabs * ((plane * esize + gran - 1) // gran) * gran      # objectness plane (upper bound by one granule)
+        # plane c of slab s starts at byte ((s*no + c)*plane*esize); its phase within a granule is one of gran/esize values
+        n_gran = (gran + plane * esize + gran - 1) // gran
         per_phase = {}
-        for phase in range(0, gran, 4):
-            if (plane * 4) % gran == 0 and phase:
+        for phase in range(0, gran, esize):
+            if (plane * esize) % gran == 0 and phase:
                 break
-            g = (phase + pos4) // gran
+            g = (phase + pos_b) // gran
             hit = torch.zeros(slabs, n_gran, dtype=torch.int32, device=h.device)
             hit.scatter_reduce_(1, g.expand(slabs, -1), loaded.int(), reduce="amax")
             per_phase[phase] = hit.sum(1)                                    # granules per slab
@@ -53,7 +54,7 @@ def touched_bytes(heads, specs, nc, conf, gran):
         for c in range(no):
             if c == 4:
                 continue
-            ph = ((sidx * no + c) * plane * 4) % gran
+            ph = ((sidx * no + c) * plane * esize) % gran
             cnt = torch.zeros(slabs, dtype=torch.int64, device=h.device)
             for phase, n in per_phase.items():
                 cnt += torch.where(ph == phase, n.long(), 0)

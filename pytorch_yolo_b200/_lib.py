@@ -42,6 +42,8 @@ class TargetLayer(C.Structure):
 ABI_VERSION = 3
 E_UNSUPPORTED = -5
 VARIANT_ACCUMULATE = 0x100
+VARIANT_F16 = 0x200
+VARIANT_BF16 = 0x400
 HEAD_ACCUMULATE = 1
 HEAD_FP32X3 = 8
 HEAD_NO_CANDIDATES = 2

@@ -27,6 +27,17 @@ __device__ __forceinline__ float4 ldg_stream4(const float* p) {
                  : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
     return v;
 }
+// 16-bit heads (fp16 / bf16 bit patterns): one element, and four consecutive elements as one 8-byte load
+__device__ __forceinline__ unsigned short ldg_stream_b16(const void* p) {
+    unsigned short v;
+    asm volatile("ld.global.nc.L1::no_allocate.b16 %0, [%1];" : "=h"(v) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ uint2 ldg_stream_b16x4(const void* p) {
+    uint2 v;
+    asm volatile("ld.global.nc.L1::no_allocate.v2.b32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p));
+    return v;
+}
 
 // max that propagates NaN (PTX max.NaN.f32, one FMNMX): a NaN anywhere poisons the running max.
 __device__ __forceinline__ float fmax_nan(float a, float b) {

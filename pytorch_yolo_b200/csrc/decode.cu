@@ -11,6 +11,10 @@
 // objectness plane whole and the box and class planes only around positions whose objectness can pass the confidence
 // threshold; decode_compact_dense_kernel (selectable) and the other kernels read every byte once.
 #include <cuda.h>          // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -19,10 +23,10 @@ namespace yb {
 // ------------------------------------------------------------------------------------------------
 // Launch-time description of one scale, derived on the host from yolo_b200_scale.
 struct ScaleDev {
-    const float* head;
+    const void* head; // fp32 elements; 16-bit elements in decode_compact's F16 / BF16 modes (LDG kernels only)
     int ny, nx, na, row_off;
     int plane;        // ny*nx
-    int vec;          // 4 when every (slab, channel) plane start is 16-byte aligned, else 1
+    int vec;          // 4 when every (slab, channel) plane start is aligned to 4 elements (16 bytes fp32, 8 bytes 16-bit), else 1
     int n_units;      // batch*na*plane / vec   work units of this scale
     int first_block;  // first blockIdx.x that works on this scale
     int first_tile;   // TMA kernel: first tile id of this scale
@@ -65,24 +69,45 @@ struct DecodeParams {
 
 constexpr int kDcThreads = YB_DC_THREADS;   // decode_compact CTA size
 
-template <int VEC>
-__device__ __forceinline__ void load_vec(float (&dst)[VEC], const float* p) {
-    if constexpr (VEC == 4) {
-        const float4 v = ldg_stream4(p);
-        dst[0] = v.x; dst[1] = v.y; dst[2] = v.z; dst[3] = v.w;
+// Head element types of the LDG decode_compact kernels: float, __half, __nv_bfloat16.  A 16-bit value is converted to fp32
+// right after the load; the conversion is exact, so everything after it is the fp32 code on the values h.float() holds.
+template <typename T> __device__ __forceinline__ float f32_of_bits(unsigned short b);
+template <> __device__ __forceinline__ float f32_of_bits<__half>(unsigned short b) { return __half2float(__ushort_as_half(b)); }
+template <> __device__ __forceinline__ float f32_of_bits<__nv_bfloat16>(unsigned short b) {
+    return __bfloat162float(__ushort_as_bfloat16(b));
+}
+__device__ __forceinline__ float to_f32(float v) { return v; }
+__device__ __forceinline__ float to_f32(__half v) { return __half2float(v); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 v) { return __bfloat162float(v); }
+
+// VEC consecutive elements at p as fp32: one 16-byte (fp32) or 8-byte (16-bit) streaming load for VEC = 4
+template <int VEC, typename T>
+__device__ __forceinline__ void load_vec(float (&dst)[VEC], const T* p) {
+    if constexpr (std::is_same_v<T, float>) {
+        if constexpr (VEC == 4) {
+            const float4 v = ldg_stream4(p);
+            dst[0] = v.x; dst[1] = v.y; dst[2] = v.z; dst[3] = v.w;
+        } else {
+            dst[0] = ldg_stream(p);
+        }
+    } else if constexpr (VEC == 4) {
+        const uint2 v = ldg_stream_b16x4(p);                       // element 0 in the low half of v.x
+        dst[0] = f32_of_bits<T>((unsigned short)(v.x & 0xffffu)); dst[1] = f32_of_bits<T>((unsigned short)(v.x >> 16));
+        dst[2] = f32_of_bits<T>((unsigned short)(v.y & 0xffffu)); dst[3] = f32_of_bits<T>((unsigned short)(v.y >> 16));
     } else {
-        dst[0] = ldg_stream(p);
+        dst[0] = f32_of_bits<T>(ldg_stream_b16(p));
     }
 }
 
 // Exact class pick in sigmoid space: first k maximising sigma(logit_k) (torch.max semantics on the
 // decoded tensor, reference utils.py:212).  Only reached when the two largest logits collapse to
 // (nearly) the same fp32 sigmoid, e.g. logits {20, 25} -> both 1.0 (SURVEY.md section 7 hard parts).
-__device__ __noinline__ void rescan_classes(const float* cls0, int stride, int nc, float& conf, int& cls) {
+template <typename T>
+__device__ __noinline__ void rescan_classes(const T* cls0, int stride, int nc, float& conf, int& cls) {
     float best = -1.0f;
     int bi = 0;
     for (int k = 0; k < nc; ++k) {
-        const float s = sigmoidf_rn(cls0[(size_t)k * stride]);       // generic load: global planes or a shared-memory tile
+        const float s = sigmoidf_rn(to_f32(cls0[(size_t)k * stride]));       // generic load: global planes or a shared-memory tile
         if (s > best) { best = s; bi = k; }
     }
     conf = best;
@@ -92,10 +117,11 @@ __device__ __noinline__ void rescan_classes(const float* cls0, int stride, int n
 // Everything after the class scan, for ONE anchor: scores, thresholds, box decode, warp-aggregated emission.
 // Shared by the LDG and the TMA kernel so that both produce bit-identical candidates.  All 32 lanes call.
 //   t0..t4   raw x, y, w, h, objectness logits          m / m2 / idx  max, second max, first arg-max class logit
-//   cls0     address of this anchor's class-0 logit, consecutive classes `cls_stride` floats apart
+//   cls0     address of this anchor's class-0 logit, consecutive classes `cls_stride` elements apart
+template <typename T>
 __device__ __forceinline__ void finish_anchor(const DecodeParams& P, const ScaleDev& S, bool active, int img, int a, int pos,
                                               float t0, float t1, float t2, float t3, float t4,
-                                              float m, float m2, int idx, const float* cls0, int cls_stride) {
+                                              float m, float m2, int idx, const T* cls0, int cls_stride) {
     const int nc = P.nc;
     const float stride = S.stride;
     const float conf = P.conf;
@@ -145,15 +171,16 @@ __device__ __forceinline__ void finish_anchor(const DecodeParams& P, const Scale
 
 // One work unit of the LDG kernels: VEC consecutive positions of one (image, anchor) slab.  Units past the end are
 // clamped onto the last one (a valid address) and marked inactive, so that the lane still takes part in the collectives.
+template <typename T>
 struct DcUnit {
-    const float* base;   // channel 0 of the unit's first position
+    const T* base;       // channel 0 of the unit's first position
     int img, a, pos0;
     bool active;
 };
 
-template <int VEC>
-__device__ __forceinline__ DcUnit dc_unit(const ScaleDev& S, int no, int unit) {
-    DcUnit u;
+template <int VEC, typename T>
+__device__ __forceinline__ DcUnit<T> dc_unit(const ScaleDev& S, int no, int unit) {
+    DcUnit<T> u;
     u.active = unit < S.n_units;
     if (!u.active) unit = S.n_units - 1;
     const int pv_per_slab = S.plane / VEC;
@@ -162,14 +189,14 @@ __device__ __forceinline__ DcUnit dc_unit(const ScaleDev& S, int no, int unit) {
     u.img = slab / S.na;
     u.a = slab - u.img * S.na;
     u.pos0 = pv * VEC;
-    u.base = S.head + (size_t)slab * no * S.plane + u.pos0;
+    u.base = static_cast<const T*>(S.head) + (size_t)slab * no * S.plane + u.pos0;
     return u;
 }
 
 // Running (max, second max, first arg-max) over the class planes at cbase, kDcUnroll planes in flight per batch; the max
 // propagates NaN.
-template <int VEC, int kDcUnroll>
-__device__ __forceinline__ void scan_classes(const float* cbase, int plane, int nc, float (&m)[VEC], float (&m2)[VEC],
+template <int VEC, int kDcUnroll, typename T>
+__device__ __forceinline__ void scan_classes(const T* cbase, int plane, int nc, float (&m)[VEC], float (&m2)[VEC],
                                              int (&idx)[VEC]) {
 #pragma unroll
     for (int j = 0; j < VEC; ++j) { m[j] = __int_as_float(0xff800000); m2[j] = m[j]; idx[j] = 0; }
@@ -213,10 +240,10 @@ __device__ __forceinline__ void scan_classes(const float* cbase, int plane, int 
 }
 
 // Dense: one unit per thread, every plane read.
-template <int VEC, int kDcUnroll>
+template <int VEC, int kDcUnroll, typename T>
 __device__ __forceinline__ void decode_compact_dense_body(const DecodeParams& P, const ScaleDev& S, int block_local) {
     const int plane = S.plane;
-    const DcUnit u = dc_unit<VEC>(S, P.nc + 5, block_local * kDcThreads + (int)threadIdx.x);
+    const DcUnit<T> u = dc_unit<VEC, T>(S, P.nc + 5, block_local * kDcThreads + (int)threadIdx.x);
 
     // box + objectness planes
     float t[5][VEC];
@@ -225,8 +252,8 @@ __device__ __forceinline__ void decode_compact_dense_body(const DecodeParams& P,
 
     float m[VEC], m2[VEC];
     int idx[VEC];
-    const float* cbase = u.base + (size_t)5 * plane;
-    scan_classes<VEC, kDcUnroll>(cbase, plane, P.nc, m, m2, idx);
+    const T* cbase = u.base + (size_t)5 * plane;
+    scan_classes<VEC, kDcUnroll, T>(cbase, plane, P.nc, m, m2, idx);
 
 #pragma unroll
     for (int j = 0; j < VEC; ++j)
@@ -250,10 +277,10 @@ __device__ __forceinline__ bool obj_gate(float t4, float conf) {
 // requested.  With every position passing, a thread issues the loads of the dense kernel, one round trip later.
 // (Variants that prefetch the objectness of a second or fourth unit per thread while scanning the current one were
 // slower on every configuration but conf 0.001: DESIGN.md section 6.)
-template <int VEC, int kDcUnroll>
+template <int VEC, int kDcUnroll, typename T>
 __device__ __forceinline__ void decode_compact_gated_body(const DecodeParams& P, const ScaleDev& S, int block_local) {
     const int plane = S.plane;
-    const DcUnit u = dc_unit<VEC>(S, P.nc + 5, block_local * kDcThreads + (int)threadIdx.x);
+    const DcUnit<T> u = dc_unit<VEC, T>(S, P.nc + 5, block_local * kDcThreads + (int)threadIdx.x);
     float t[5][VEC];
     load_vec<VEC>(t[4], u.base + (size_t)4 * plane);
     bool gate[VEC];
@@ -265,11 +292,11 @@ __device__ __forceinline__ void decode_compact_gated_body(const DecodeParams& P,
     }
     float m[VEC], m2[VEC];
     int idx[VEC];
-    const float* cbase = u.base + (size_t)5 * plane;
+    const T* cbase = u.base + (size_t)5 * plane;
     if (any) {
 #pragma unroll
         for (int c = 0; c < 4; ++c) load_vec<VEC>(t[c], u.base + (size_t)c * plane);
-        scan_classes<VEC, kDcUnroll>(cbase, plane, P.nc, m, m2, idx);
+        scan_classes<VEC, kDcUnroll, T>(cbase, plane, P.nc, m, m2, idx);
     } else {                                                   // finish_anchor reads none of these for a gated-off position
 #pragma unroll
         for (int j = 0; j < VEC; ++j) {
@@ -292,20 +319,23 @@ __device__ __forceinline__ const ScaleDev& dc_scale(const DecodeParams& P) {
     return P.sc[s];
 }
 
+// T: the element type of every head of the launch (float, __half, __nv_bfloat16)
+template <typename T>
 __global__ void __launch_bounds__(kDcThreads, YB_DC_MINBLOCKS)
 decode_compact_kernel(const __grid_constant__ DecodeParams P) {
     const ScaleDev& S = dc_scale(P);
     const int block_local = (int)blockIdx.x - S.first_block;
-    if (S.vec == 4) decode_compact_gated_body<4, YB_DC_UNROLL>(P, S, block_local);
-    else            decode_compact_gated_body<1, YB_DC_UNROLL1>(P, S, block_local);
+    if (S.vec == 4) decode_compact_gated_body<4, YB_DC_UNROLL, T>(P, S, block_local);
+    else            decode_compact_gated_body<1, YB_DC_UNROLL1, T>(P, S, block_local);
 }
 
+template <typename T>
 __global__ void __launch_bounds__(kDcThreads, YB_DC_MINBLOCKS)
 decode_compact_dense_kernel(const __grid_constant__ DecodeParams P) {
     const ScaleDev& S = dc_scale(P);
     const int block_local = (int)blockIdx.x - S.first_block;
-    if (S.vec == 4) decode_compact_dense_body<4, YB_DC_UNROLL>(P, S, block_local);
-    else            decode_compact_dense_body<1, YB_DC_UNROLL1>(P, S, block_local);
+    if (S.vec == 4) decode_compact_dense_body<4, YB_DC_UNROLL, T>(P, S, block_local);
+    else            decode_compact_dense_body<1, YB_DC_UNROLL1, T>(P, S, block_local);
 }
 
 // ---- mbarrier / TMA bulk-copy helpers --------------------------------------------------------------
@@ -407,7 +437,7 @@ decode_compact_tma_kernel(const __grid_constant__ DecodeParams P) {
             const uint32_t bytes = (uint32_t)np * 4u;
             if (lane == 0) mbar_expect_tx(&full[st], bytes * (uint32_t)no);
             __syncwarp();
-            const float* src = S.head + (size_t)slab * no * S.plane + p0;
+            const float* src = static_cast<const float*>(S.head) + (size_t)slab * no * S.plane + p0;
             for (int c = lane; c < no; c += 32)
                 tma_bulk_g2s(dst + (size_t)c * tp, src + (size_t)c * S.plane, bytes, &full[st]);
         }
@@ -431,7 +461,7 @@ decode_compact_tma_kernel(const __grid_constant__ DecodeParams P) {
             full_parity ^= 1u << st;
         } else {
             consumer_bar_sync();                                       // nobody still reads this stage
-            const float* src = S.head + (size_t)slab * no * S.plane + p0;
+            const float* src = static_cast<const float*>(S.head) + (size_t)slab * no * S.plane + p0;
             // a warp copies one channel row at a time, 8 loads in flight per lane
             for (int c = tid >> 5; c < no; c += kTcConsumers / 32) {
                 const float* row = src + (size_t)c * S.plane;
@@ -510,7 +540,7 @@ decode_dense_kernel(const __grid_constant__ DecodeParams P) {
         // which makes the 32 addresses of one store hit 32 different banks (row pitch 5+nc is odd).
         const int warp = (int)threadIdx.x >> 5, lane = (int)threadIdx.x & 31, g = lane >> 3;
         if (4 * lane < np) {
-            const float* src = S.head + (size_t)slab * no * plane + p0 + 4 * lane;
+            const float* src = static_cast<const float*>(S.head) + (size_t)slab * no * plane + p0 + 4 * lane;
             const float stride = S.stride;
             float* drow[4];
 #pragma unroll
@@ -568,7 +598,7 @@ decode_dense_kernel(const __grid_constant__ DecodeParams P) {
         const int n_sig = no - 4;
         const int n0 = n_sig > 4 ? (n_sig - 4) / 2 : 0;
         if (p < np) {
-            const float* src = S.head + (size_t)slab * no * plane + p0 + p;
+            const float* src = static_cast<const float*>(S.head) + (size_t)slab * no * plane + p0 + p;
             float* dst = tl + p * no;
             const float stride = S.stride;
             if (half == 0) {
@@ -880,8 +910,9 @@ static cudaError_t zero_counters(int32_t* count, int32_t* overflow, int batch, c
     return cudaMemsetAsync(overflow, 0, sizeof(int32_t), stream);
 }
 
+// esize: bytes per head element (4, or 2 for decode_compact's 16-bit modes)
 static int fill_params(DecodeParams& P, const yolo_b200_scale* sc, int n_scales, int batch, int nc,
-                       int rows_per_img, bool dense, bool partial = false) {
+                       int rows_per_img, bool dense, bool partial = false, int esize = 4) {
     if (!sc) return YOLO_B200_E_NULL;
     if (n_scales < 1 || n_scales > YOLO_B200_MAX_SCALES || batch < 0 || nc < 1 || nc > YOLO_B200_MAX_CLASSES ||
         rows_per_img < 1)
@@ -893,13 +924,14 @@ static int fill_params(DecodeParams& P, const yolo_b200_scale* sc, int n_scales,
         ScaleDev& d = P.sc[k];
         if (!s.head && batch > 0) return YOLO_B200_E_NULL;
         if (s.ny < 1 || s.nx < 1 || s.na < 1 || s.na > YOLO_B200_MAX_ANCHORS || s.row_off < 0) return YOLO_B200_E_RANGE;
-        if (((uintptr_t)s.head & 3u) != 0) return YOLO_B200_E_ALIGN;
+        if (((uintptr_t)s.head & (uintptr_t)(esize - 1)) != 0) return YOLO_B200_E_ALIGN;
         d.head = s.head; d.ny = s.ny; d.nx = s.nx; d.na = s.na; d.row_off = s.row_off;
         d.plane = s.ny * s.nx;
         d.stride = s.stride;
         for (int a = 0; a < YOLO_B200_MAX_ANCHORS; ++a) { d.av[a][0] = s.anchor_vec[a][0]; d.av[a][1] = s.anchor_vec[a][1]; }
-        // every plane starts at head + (slab*no + c)*plane floats: 16-byte aligned for all (slab, c) iff plane % 4 == 0
-        d.vec = ((d.plane % 4 == 0) && (((uintptr_t)s.head & 15u) == 0)) ? 4 : 1;
+        // every plane starts at head + (slab*no + c)*plane elements: aligned to 4 elements for all (slab, c) iff
+        // plane % 4 == 0 and head is
+        d.vec = ((d.plane % 4 == 0) && (((uintptr_t)s.head & (uintptr_t)(4 * esize - 1)) == 0)) ? 4 : 1;
         const long long slabs = (long long)batch * s.na;
         if ((long long)s.row_off + (long long)s.na * d.plane > rows_per_img) return YOLO_B200_E_RANGE;
         if (slabs * d.plane > 0x7fffffffLL) return YOLO_B200_E_RANGE;
@@ -992,11 +1024,15 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     if (!cand_box || !cand_meta || !count || !overflow) return YOLO_B200_E_NULL;
     const bool accumulate = variant >= 0 && (variant & YOLO_B200_VARIANT_ACCUMULATE) != 0;
     if (accumulate) variant &= ~YOLO_B200_VARIANT_ACCUMULATE;
+    const int half_bits = variant >= 0 ? variant & (YOLO_B200_VARIANT_F16 | YOLO_B200_VARIANT_BF16) : 0;
+    variant &= ~half_bits;
     if (cap_per_img < 1 || variant < 0 || variant > 4) return YOLO_B200_E_RANGE;
+    if (half_bits == (YOLO_B200_VARIANT_F16 | YOLO_B200_VARIANT_BF16)) return YOLO_B200_E_RANGE;
+    if (half_bits && (variant == 2 || variant == 3)) return YOLO_B200_E_UNSUPPORTED;     // the TMA kernels read fp32 only
     if ((((uintptr_t)cand_box) | ((uintptr_t)cand_meta)) & 15u) return YOLO_B200_E_ALIGN;
     const bool gated = variant <= 1;
     DecodeParams P{};
-    const int blocks = fill_params(P, scales, n_scales, batch, nc, rows_per_img, false, accumulate);
+    const int blocks = fill_params(P, scales, n_scales, batch, nc, rows_per_img, false, accumulate, half_bits ? 2 : 4);
     if (blocks < 0) return blocks;
     P.conf = conf_thres; P.min_wh = min_wh;
     P.cand_box = cand_box; P.cand_meta = cand_meta; P.cap = cap_per_img; P.count = count; P.overflow = overflow;
@@ -1027,10 +1063,16 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
             return (int)e;
         const int grid = (int)(tiles < sms ? tiles : sms);
         decode_compact_tma_kernel<<<grid, kTcThreads, smem, stream>>>(P);
+    } else if (half_bits == YOLO_B200_VARIANT_F16) {
+        if (gated) decode_compact_kernel<__half><<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
+        else       decode_compact_dense_kernel<__half><<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
+    } else if (half_bits == YOLO_B200_VARIANT_BF16) {
+        if (gated) decode_compact_kernel<__nv_bfloat16><<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
+        else       decode_compact_dense_kernel<__nv_bfloat16><<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
     } else if (gated) {
-        decode_compact_kernel<<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
+        decode_compact_kernel<float><<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
     } else {
-        decode_compact_dense_kernel<<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
+        decode_compact_dense_kernel<float><<<blocks, kDcThreads, YB_DC_SMEM_PAD, stream>>>(P);
     }
     return (int)cudaGetLastError();
 }

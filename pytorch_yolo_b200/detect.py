@@ -119,13 +119,14 @@ class Detector:
         with torch.cuda.graph(g):          # the side stream forks from / joins torch's capture stream: one graph, two priorities
             self._enqueue(inputs)
         self._graph = g
-        self._bound = (tuple(h.data_ptr() for h in inputs), inputs)
+        self._bound = (tuple((h.data_ptr(), h.dtype) for h in inputs), inputs)
 
     def launch(self, inputs: Sequence[torch.Tensor]) -> None:
         """Enqueue one step on the current stream (no host sync)."""
         self._stream = torch.cuda.current_stream(self.device)
         if self.use_graph:
-            ptrs = tuple(h.data_ptr() for h in inputs)
+            # the dtype picks the kernel: a 16-bit tensor at a freed fp32 tensor's address needs a new graph
+            ptrs = tuple((h.data_ptr(), h.dtype) for h in inputs)
             if self._bound is None or self._bound[0] != ptrs:
                 self.bind(inputs)
             self._graph.replay()
@@ -176,7 +177,7 @@ class Detector:
         h2d = 0
         for d, h in zip(dev_heads, host_heads):
             d.copy_(h, non_blocking=True)
-            h2d += h.numel() * 4
+            h2d += h.numel() * h.element_size()
         self.launch(dev_heads)
         _, kept = self.counts()
         n_max = int(kept.max()) if self.batch else 0

@@ -19,14 +19,27 @@ MIN_WH = 2.0           # reference utils/utils.py:207
 MAX_PER_CLASS = 100    # reference utils/utils.py:247-250
 
 
+_FP32 = (torch.float32,)
+# head dtypes decode_compact reads, and the variant bit that tells the library (include/yolo_b200.h)
+HEAD_DTYPE_BITS = {torch.float32: 0, torch.float16: _lib.VARIANT_F16, torch.bfloat16: _lib.VARIANT_BF16}
+
+
 def _require_cuda(t: torch.Tensor, what: str) -> None:
+    _require_device(t, what)
+    _require_dtype(t, what, _FP32)
+
+
+def _require_device(t: torch.Tensor, what: str) -> None:
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{what}: expected a torch.Tensor, got {type(t).__name__}")
     if not t.is_cuda:
         raise YoloB200Error(f"{what} is on {t.device}: pytorch_yolo_b200 has no CPU path "
                             "(the kernels are sm_100a CUDA); move the tensor to a CUDA device")
-    if t.dtype != torch.float32:
-        raise TypeError(f"{what}: expected float32, got {t.dtype}")
+
+
+def _require_dtype(t: torch.Tensor, what: str, dtypes) -> None:
+    if t.dtype not in dtypes:
+        raise TypeError(f"{what}: expected {' or '.join(str(d).replace('torch.', '') for d in dtypes)}, got {t.dtype}")
 
 
 def _stream_ptr(device) -> int:
@@ -59,7 +72,7 @@ def scale_spec(anchors, ny: int, nx: int, img_size) -> ScaleSpec:
     return ScaleSpec(tuple((float(a), float(b)) for a, b in anchors), int(ny), int(nx), float(stride), vec)
 
 
-def _fill_scales(heads: Sequence[torch.Tensor], specs: Sequence[ScaleSpec], nc: int):
+def _fill_scales(heads: Sequence[torch.Tensor], specs: Sequence[ScaleSpec], nc: int, dtypes=_FP32):
     if not 1 <= len(heads) <= MAX_SCALES or len(heads) != len(specs):
         raise ValueError(f"need 1..{MAX_SCALES} heads with one spec each, got {len(heads)} / {len(specs)}")
     arr = (Scale * len(heads))()
@@ -68,9 +81,12 @@ def _fill_scales(heads: Sequence[torch.Tensor], specs: Sequence[ScaleSpec], nc: 
     row_off = 0
     keep = []
     for k, (h, sp) in enumerate(zip(heads, specs)):
-        _require_cuda(h, f"head {k}")
+        _require_device(h, f"head {k}")
+        _require_dtype(h, f"head {k}", dtypes)
         if h.device != dev or h.shape[0] != batch:
             raise ValueError("all heads must share device and batch size")
+        if h.dtype != heads[0].dtype:
+            raise ValueError(f"all heads of one call must share a dtype: head 0 is {heads[0].dtype}, head {k} {h.dtype}")
         if h.dim() != 4 or h.shape[1] != sp.na * (nc + 5) or h.shape[2] != sp.ny or h.shape[3] != sp.nx:
             raise ValueError(f"head {k}: expected (B, {sp.na * (nc + 5)}, {sp.ny}, {sp.nx}), got {tuple(h.shape)}")
         if not h.is_contiguous():
@@ -175,11 +191,14 @@ def decode_compact(heads, specs, nc: int, conf_thres: float, buf: Buffers, min_w
                    variant: str = "auto", row_offs: Optional[Sequence[int]] = None,
                    rows_per_img: Optional[int] = None, accumulate: bool = False) -> None:
     """Fused decode + filter + compaction into ``buf`` (no (B, N, 5+nc) tensor is materialised).
+    ``heads``: float32, float16 or bfloat16, one dtype for all.  16-bit heads are converted to fp32 as the kernel loads
+    them, so the candidates are bit-identical to those of ``[h.float() for h in heads]``; the TMA variants read float32
+    only.
     ``variant``: "auto" | "ldg" | "tma" | "tma2d" | "ldg_dense" (identical results; see include/yolo_b200.h).
     ``row_offs`` / ``rows_per_img`` / ``accumulate``: decode only some scales of a model and append to the candidates
     already in ``buf`` (the other scales went through :func:`head_decode_compact`)."""
     lib = _lib.load()
-    arr, keep, batch, rows, dev = _fill_scales(heads, specs, nc)
+    arr, keep, batch, rows, dev = _fill_scales(heads, specs, nc, tuple(HEAD_DTYPE_BITS))
     if row_offs is not None:
         for k, off in enumerate(row_offs):
             arr[k].row_off = int(off)
@@ -190,7 +209,8 @@ def decode_compact(heads, specs, nc: int, conf_thres: float, buf: Buffers, min_w
         check(lib.yolo_b200_decode_compact_ex(arr, len(keep), batch, nc, rows, conf_thres, min_wh,
                                               buf.cand_box.data_ptr(), buf.cand_meta.data_ptr(), buf.cap,
                                               buf.count_ptr, buf.overflow_ptr,
-                                              DECODE_VARIANTS[variant] | (_lib.VARIANT_ACCUMULATE if accumulate else 0),
+                                              DECODE_VARIANTS[variant] | (_lib.VARIANT_ACCUMULATE if accumulate else 0)
+                                              | HEAD_DTYPE_BITS[keep[0].dtype],
                                               _stream_ptr(dev)),
               "yolo_b200_decode_compact")
 

@@ -9,6 +9,12 @@ Documented behaviour where the reference is undefined:
 * score ties keep ascending anchor-row order (the reference's argsort is unstable);
 * ``nms_thres >= 1`` raises ``ValueError`` (the reference loops forever);
 * tensors must be float32 on a CUDA device -- there is no CPU path.
+
+The fused path (``detect``, ``detect_layers``, ``Detector``, ``PipelinedDetector``, ``ShardedDetector``, ``EvalPipeline``)
+also takes fp16 and bf16 head tensors, as a ``.half()`` or autocast model produces them, and decodes them in fp32: the
+results are bit-identical to those from ``[h.float() for h in heads]``.  That deviates from the reference on 16-bit
+input, which computes ``io`` in 16 bits and rounds after every op (box corners at 608 px carry ulps of 0.25-0.5 px).
+``non_max_suppression``, ``decode_layers`` and ``YOLOLayer.forward`` keep taking float32 only.
 """
 from __future__ import annotations
 
