@@ -43,3 +43,22 @@ def assert_dets_equal(got, want, box_rtol=0.0, what=""):
                 f"(max abs {float((g[:, :4] - w[:, :4]).abs().max()):.3e})"
         else:
             torch.testing.assert_close(g[:, :4], w[:, :4], rtol=box_rtol, atol=1e-30, msg=lambda m: f"{what} image {i}: {m}")
+
+
+def prediction_with_class_sizes(sizes_per_image, nc, seed):
+    """(B, N, 5+nc) decoded-looking tensor in which class c of image b holds exactly sizes_per_image[b][c] candidates
+    (boxes clustered so that suppression and MERGE clusters occur), rows shuffled."""
+    g = torch.Generator().manual_seed(seed)
+    n = max(sum(s) for s in sizes_per_image)
+    pred = torch.zeros(len(sizes_per_image), n, 5 + nc)
+    for b, sizes in enumerate(sizes_per_image):
+        cls = torch.cat([torch.full((k,), c, dtype=torch.long) for c, k in enumerate(sizes)])
+        m = len(cls)
+        centre = 300 * torch.rand(nc, 2, generator=g) + 100
+        pred[b, :m, 0:2] = centre[cls] + 12 * torch.randn(m, 2, generator=g)
+        pred[b, :m, 2:4] = 40 + 25 * torch.rand(m, 2, generator=g)
+        pred[b, :m, 4] = 0.3 + 0.7 * torch.rand(m, generator=g)
+        pred[b, torch.arange(m), 5 + cls] = 0.5 + 0.5 * torch.rand(m, generator=g)
+        perm = torch.randperm(n, generator=g)
+        pred[b] = pred[b, perm]                       # rows beyond m are all-zero: score 0, dropped by the filter
+    return pred

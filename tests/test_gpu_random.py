@@ -7,7 +7,7 @@ import torch
 
 from oracle import yolo_oracle
 from pytorch_yolo_b200 import YOLOLayer, decode_layers, detect_layers, non_max_suppression, synth
-from tests.helpers import assert_dets_equal
+from tests.helpers import assert_dets_equal, prediction_with_class_sizes
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -116,25 +116,6 @@ def test_dense_decode_tma_equals_ldg(nc, grids, batch):
     assert torch.equal(outs["ldg"], outs["tma"])
 
 
-def _prediction_with_class_sizes(sizes_per_image, nc, seed):
-    """(B, N, 5+nc) decoded-looking tensor in which class c of image b holds exactly sizes_per_image[b][c] candidates
-    (boxes clustered so that suppression and MERGE clusters occur), rows shuffled."""
-    g = torch.Generator().manual_seed(seed)
-    n = max(sum(s) for s in sizes_per_image)
-    pred = torch.zeros(len(sizes_per_image), n, 5 + nc)
-    for b, sizes in enumerate(sizes_per_image):
-        cls = torch.cat([torch.full((k,), c, dtype=torch.long) for c, k in enumerate(sizes)])
-        m = len(cls)
-        centre = 300 * torch.rand(nc, 2, generator=g) + 100
-        pred[b, :m, 0:2] = centre[cls] + 12 * torch.randn(m, 2, generator=g)
-        pred[b, :m, 2:4] = 40 + 25 * torch.rand(m, 2, generator=g)
-        pred[b, :m, 4] = 0.3 + 0.7 * torch.rand(m, generator=g)
-        pred[b, torch.arange(m), 5 + cls] = 0.5 + 0.5 * torch.rand(m, generator=g)
-        perm = torch.randperm(n, generator=g)
-        pred[b] = pred[b, perm]                       # rows beyond m are all-zero: score 0, dropped by the filter
-    return pred
-
-
 def test_packed_groups_mixed_class_sizes():
     """The segment stage's two work lists in one call: empty, single-box, small (packed several to a warp, runs that end
     at 8-class block borders, exactly 32 lanes), 33..64, 65..128 and capped (> 100) classes interleaved -- bit-exact
@@ -146,7 +127,7 @@ def test_packed_groups_mixed_class_sizes():
         [16, 16, 16, 16, 1, 0, 17, 15, 2, 2, 2, 2, 2, 2, 2, 2, 8, 8, 8, 8, 65],
         [0] * 20 + [2],
     ]
-    pred_cpu = _prediction_with_class_sizes(sizes, nc, seed=11)
+    pred_cpu = prediction_with_class_sizes(sizes, nc, seed=11)
     want, wrows = yolo_oracle.non_max_suppression_indexed(pred_cpu.clone(), 0.05, 0.45)
     got, rows = non_max_suppression(pred_cpu.clone().to(DEV), 0.05, 0.45, return_rows=True)
     assert_dets_equal(got, want, box_rtol=1e-5, what="mixed class sizes")
@@ -161,7 +142,7 @@ def test_small_max_per_class_turns_packing_off(mpc, monkeypatch):
     from pytorch_yolo_b200 import ops
     nc = 12
     sizes = [[0, 1, 2, 4, 6, 20, 31, 32, 33, 50, 3, 3], [7] * 12]
-    pred_cpu = _prediction_with_class_sizes(sizes, nc, seed=mpc)
+    pred_cpu = prediction_with_class_sizes(sizes, nc, seed=mpc)
     monkeypatch.setattr(yolo_oracle, "MAX_PER_CLASS", mpc)
     want, wrows = yolo_oracle.non_max_suppression_indexed(pred_cpu.clone(), 0.05, 0.5)
     pred = pred_cpu.clone().to(DEV)
