@@ -76,7 +76,9 @@ int yolo_b200_decode_dense(const yolo_b200_scale* scales_host, int n_scales, int
                            int rows_per_img, float* io, yolo_b200_stream_t stream);
 /* Same call with an explicit kernel variant: 0 = automatic, 1 = LDG kernel (one CTA per 128-position tile, load phase then
  * store phase), 2 = TMA kernel (persistent CTAs: tensor-map tile loads into a shared-memory ring, transposed tiles leave
- * as bulk copies shared -> global; needs 5+n_classes <= 147).  Identical results. */
+ * as bulk copies shared -> global; needs 5+n_classes <= 150).  Identical results.  Automatic picks the TMA kernel for
+ * the scales whose planes are a multiple of 4 floats when 5+n_classes <= 150, the LDG kernel for everything else.  A call
+ * refused with an argument error (YOLO_B200_E_*) enqueues nothing: io keeps what it held. */
 int yolo_b200_decode_dense_ex(const yolo_b200_scale* scales_host, int n_scales, int batch, int n_classes,
                               int rows_per_img, float* io, int variant, yolo_b200_stream_t stream);
 
@@ -92,9 +94,10 @@ int yolo_b200_decode_compact(const yolo_b200_scale* scales_host, int n_scales, i
 
 /* Same call with an explicit kernel variant: 0 = automatic (= 1), 1 = gated LDG kernel (many small CTAs, 128-bit
  * coalesced loads; reads the objectness plane first and the box and class planes only around positions whose objectness
- * can pass conf_thres), 2 = TMA kernel (persistent CTAs, ring of 1-D cp.async.bulk copies), 3 = the same kernel fed by one
- * 2-D tensor-map copy per tile (needs 5+n_classes <= 256), 4 = dense LDG kernel (variant 1 without the gate: reads every
- * plane).  Variants 2 to 4 read the whole head tensor.  All produce identical candidates. */
+ * can pass conf_thres), 2 = TMA kernel (persistent CTAs, ring of 1-D cp.async.bulk copies; needs 5+n_classes <= 800),
+ * 3 = the same kernel fed by one 2-D tensor-map copy per tile (needs 5+n_classes <= 256), 4 = dense LDG kernel (variant 1
+ * without the gate: reads every plane).  Variants 2 to 4 read the whole head tensor.  All produce identical candidates.
+ * A call refused with an argument error (YOLO_B200_E_*) enqueues nothing: count and overflow keep what they held. */
 int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales_host, int n_scales, int batch, int n_classes,
                                 int rows_per_img, float conf_thres, float min_wh,
                                 yolo_b200_box* cand_box, yolo_b200_meta* cand_meta, int cap_per_img,

@@ -979,7 +979,8 @@ static int tma_tile_positions(int no) {
 }
 
 // Tile table (first_tile, tiles_per_slab, n_tiles) for tiles of `tp` positions, and -- with_maps -- one 2-D tensor map
-// [plane positions] x [batch*na*(5+nc) channel rows], box = [tp] x [5+nc], per scale with 16-byte aligned planes.
+// [plane positions] x [batch*na*(5+nc) channel rows], box = [tp] x [5+nc], per scale with 16-byte aligned planes.  A TMA
+// box is at most 256 rows: callers asking for maps keep 5+nc <= 256.
 static int tile_table(DecodeParams& P, int n_scales, int batch, int no, int tp, bool with_maps, bool aligned_only = false) {
     long long tiles = 0;
     P.tp = tp;
@@ -994,7 +995,6 @@ static int tile_table(DecodeParams& P, int n_scales, int batch, int no, int tp, 
     if (tiles > 0x7fffffffLL) return YOLO_B200_E_RANGE;
     P.n_tiles = (int)tiles;
     if (!with_maps) return 0;
-    if (no > 256) return YOLO_B200_E_RANGE;                             // a TMA box is at most 256 rows
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -1036,12 +1036,6 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     if (blocks < 0) return blocks;
     P.conf = conf_thres; P.min_wh = min_wh;
     P.cand_box = cand_box; P.cand_meta = cand_meta; P.cap = cap_per_img; P.count = count; P.overflow = overflow;
-    cudaError_t e;
-    if (!accumulate && (e = zero_counters(count, overflow, batch, stream)) != cudaSuccess) return (int)e;
-    if (blocks == 0) return 0;
-
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int no = nc + 5;
     const int tp = tma_tile_positions(no);
     // Measured on B200 (profiles/r01_c_decode_variants.txt): the dense LDG kernel streams at 5.8 TB/s, the 1-D bulk-copy
@@ -1049,7 +1043,15 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     // LDG kernel reads box and class planes only where the objectness can pass (profiles/gated_decode_probe.txt).  The
     // others stay selectable for comparison (2 = 1-D bulk copies, 3 = one 2-D tensor-map copy per tile, 4 = dense LDG).
     const bool use_tma = variant == 2 || variant == 3;
+    // refusals come before the counters are zeroed: a refused call must leave the counts of an earlier call intact
     if (use_tma && tp == 0) return YOLO_B200_E_RANGE;
+    if (variant == 3 && no > 256) return YOLO_B200_E_RANGE;            // a TMA box is at most 256 rows
+    cudaError_t e;
+    if (!accumulate && (e = zero_counters(count, overflow, batch, stream)) != cudaSuccess) return (int)e;
+    if (blocks == 0) return 0;
+
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     P.use_tmap = 0;
     if (use_tma) {
         const int rc = tile_table(P, n_scales, batch, no, tp, variant == 3);

@@ -17,6 +17,7 @@ import torch
 from torch import nn
 
 from pytorch_yolo_b200 import ops
+from tests.helpers import assert_same_candidates, expected_candidates, read_candidates
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -321,52 +322,6 @@ def class_logits(heads, specs, nc):
         b = h.shape[0]
         parts.append(h.detach().cpu().view(b, s.na, 5 + nc, s.ny * s.nx)[:, :, 5:].permute(0, 1, 3, 2).reshape(b, -1, nc))
     return torch.cat(parts, 1).numpy()
-
-
-def expected_candidates(dense, conf, min_wh=ops.MIN_WH):
-    """Per image: (rows, meta (score, cls_conf bits; class; row), box bits) of what the reference emits on the decoded
-    tensor: first arg-max of the sigmoid columns, score = fl(sigma(obj) * cls_conf)."""
-    d = dense.cpu().numpy()
-    with np.errstate(invalid="ignore", over="ignore"):
-        cls_s = d[..., 5:]
-        cls = np.argmax(cls_s, -1)
-        cls_conf = np.take_along_axis(cls_s, cls[..., None], -1)[..., 0]
-        score = d[..., 4] * cls_conf
-        x, y, w, h = d[..., 0], d[..., 1], d[..., 2], d[..., 3]
-        emit = (~np.isnan(d).any(-1)) & (score > np.float32(conf)) & (w > np.float32(min_wh)) & (h > np.float32(min_wh))
-        emit &= np.isfinite(d[..., :4]).all(-1)
-        hw, hh = w * np.float32(0.5), h * np.float32(0.5)
-        box = np.stack([x - hw, y - hh, x + hw, y + hh], -1)
-    per_img = []
-    for b in range(d.shape[0]):
-        r = np.nonzero(emit[b])[0]
-        meta = np.stack([score[b, r].view(np.int32), cls_conf[b, r].view(np.int32), cls[b, r].astype(np.int32),
-                         r.astype(np.int32)], -1)
-        per_img.append((meta, box[b, r].view(np.int32)))
-    return per_img, emit, cls
-
-
-def read_candidates(buf):
-    counts, _, ovf = ops.read_counts(buf)
-    assert ovf == 0
-    counts = counts.clone()
-    out = []
-    for b in range(buf.batch):
-        n = int(counts[b])
-        meta = buf.cand_meta[b * buf.cap:b * buf.cap + n].cpu().numpy()
-        box = buf.cand_box[b * buf.cap:b * buf.cap + n].cpu().numpy().view(np.int32)
-        o = np.argsort(meta[:, 3], kind="stable")
-        out.append((meta[o], box[o]))
-    return out
-
-
-def assert_same_candidates(got, want, what):
-    for b, ((gm, gb), (wm, wb)) in enumerate(zip(got, want)):
-        assert gm.shape == wm.shape, f"{what} image {b}: {len(gm)} candidates, expected {len(wm)}"
-        bad = np.nonzero((gm != wm).any(-1) | (gb != wb).any(-1))[0]
-        assert bad.size == 0, (f"{what} image {b}: {bad.size} candidates differ, first row {wm[bad[0], 3]}: "
-                               f"got class {gm[bad[0], 2]} conf {gm[bad[0], 1:2].view(np.float32)}, expected class "
-                               f"{wm[bad[0], 2]} conf {wm[bad[0], 1:2].view(np.float32)}")
 
 
 def assert_reach_and_fp64(dense, logits, emit, cls, nc, what):
