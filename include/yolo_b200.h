@@ -161,14 +161,19 @@ int yolo_b200_nms_ex(const yolo_b200_box* cand_box, const yolo_b200_meta* cand_m
  * the accumulator: the (B, na*(5+nc), ny, nx) head tensor never reaches HBM unless head_out asks for it.
  * The caller folds an eval-mode BatchNorm into weight/bias (what ConvBlock.fuse does, models/yolo_base.py:46-57). */
 typedef struct {
-    const float* x;          /* (B, c_in, ny, nx) fp32 NCHW contiguous, 16-byte aligned: input of the head convolution */
+    const float* x;          /* (B, c_in, ny, nx) fp32 NCHW contiguous, 16-byte aligned: input of the head convolution.
+                                With YOLO_B200_HEAD_F16 / _BF16: fp16 / bf16 elements, (B, c_in, pitch) */
     const float* weight;     /* (256, c_in) fp32 row-major, 16-byte aligned: rows na*(5+nc) .. 255 zero (the kernel's W tile
                                 covers up to 256 output channels; which rows it fetches depends on the instantiation);
-                                (512, c_in) with YOLO_B200_HEAD_FP32X3 */
+                                (512, c_in) with YOLO_B200_HEAD_FP32X3; (256, c_in) of x's 16-bit type with YOLO_B200_HEAD_F16 /
+                                _BF16 */
     const float* bias_host;  /* HOST pointer: na*(5+nc) floats */
     float* head_out;         /* optional: (B, na*(5+nc), ny, nx) activated head tensor (what YOLOLayer.forward receives), or NULL */
-    int32_t c_in;            /* multiple of 32 */
-    int32_t x_row_pitch;     /* floats between consecutive channel planes of x; 0 = ny*nx (contiguous NCHW).  When given it must be
+    int32_t c_in;            /* multiple of 32 (16-bit x: of 64) */
+    int32_t x_row_pitch;     /* elements between consecutive channel planes of x; 0 = ny*nx (contiguous NCHW).  16-bit x: when
+                                given, a multiple of 8 (a 16-byte row pitch); contiguous planes that are not a multiple of 8
+                                elements are read in place when even (38x38, 26x26, 19x20 ...), odd ones (19x19, 13x13) need
+                                the padded copy of yolo_b200_pad_planes_16.  fp32 x: when given it must be
                                 a multiple of 4 (TMA row pitch of 16 bytes).  A contiguous 19x19 or 13x13 map (361 / 169 floats
                                 per plane) has no such pitch: the one-pass single-CTA kernel reads it in place with loader warps
                                 (4-byte asynchronous copies); the three-pass mode and the CTA-pair kernel take it as a
@@ -186,6 +191,15 @@ typedef struct {
                                             `weight` then holds 512 rows -- rows 256 .. 511 = w - trunc_tf32(w) of rows 0 .. 255,
                                             trunc_tf32 = clear the low 13 mantissa bits -- and the head tensor matches an fp32
                                             convolution to accumulation accuracy (about three times the tensor time) */
+/* flags: x and weight hold fp16 (F16) or bf16 (BF16) elements.  The products run on tcgen05.mma kind::f16 (exact products of
+ * the 16-bit operands, fp32 accumulation); bias, activation, decode and head_out stay fp32, and the candidates are
+ * bit-identical to yolo_b200_decode_compact on the head tensor the same call writes to head_out.  One-pass single-CTA
+ * kernel only; every return code is decided before anything is enqueued (count and overflow keep what they held):
+ *   both bits: YOLO_B200_E_RANGE;  either bit with YOLO_B200_HEAD_FP32X3 or _CTA_PAIR: YOLO_B200_E_UNSUPPORTED;
+ *   c_in % 64 != 0, an odd contiguous plane, or an x_row_pitch that is not a multiple of 8: YOLO_B200_E_UNSUPPORTED;
+ *   x or weight not 16-byte aligned: YOLO_B200_E_ALIGN. */
+#define YOLO_B200_HEAD_F16           0x10
+#define YOLO_B200_HEAD_BF16          0x20
 #define YOLO_B200_HEAD_PROFILE_MAINLOOP 0x100  /* flags, profiling only (results are garbage): skip the epilogue */
 #define YOLO_B200_HEAD_PROFILE_NO_W     0x200  /* profiling only: the weight tiles are fetched once, not per position tile */
 #define YOLO_B200_HEAD_PROFILE_NO_X     0x400  /* profiling only: the feature tiles are fetched once */
@@ -195,13 +209,18 @@ typedef struct {
  * whose planes are not a multiple of 4 floats (19x19, 13x13) the 16-byte row pitch the fused head kernel's TMA loads need.
  * x 4-byte aligned, out 16-byte aligned. */
 int yolo_b200_pad_planes(const float* x, float* out, long long rows, int plane, int pitch, yolo_b200_stream_t stream);
+/* The same for 2-byte elements (fp16 / bf16 feature maps): (rows, plane) -> (rows, pitch), pitch >= plane and pitch % 8 == 0,
+ * pad columns zero.  x 2-byte aligned, out 16-byte aligned. */
+int yolo_b200_pad_planes_16(const void* x, void* out, long long rows, int plane, int pitch, yolo_b200_stream_t stream);
 
 /* 1 when the fused kernel covers this geometry: c_in % 32 == 0, a row pitch x_row_pitch % 4 == 0 or contiguous planes, and
  * 3 anchors with 3*(5+n_classes) <= 256 (80, 20 and 1 classes have fully unrolled epilogues, any other count up to 80
  * runs a kernel with a run-time class loop).  Other scales go through the caller's own convolution +
  * yolo_b200_decode_compact_ex(... | YOLO_B200_VARIANT_ACCUMULATE). */
 int yolo_b200_head_supported(int c_in, int ny, int nx, int x_row_pitch, int na, int n_classes);
-/* the same question for a call with `flags` (YOLO_B200_HEAD_FP32X3, YOLO_B200_HEAD_CTA_PAIR: those need a 16-byte row pitch) */
+/* the same question for a call with `flags` (YOLO_B200_HEAD_FP32X3, YOLO_B200_HEAD_CTA_PAIR: those need a 16-byte row pitch;
+ * YOLO_B200_HEAD_F16 / _BF16: c_in % 64 == 0 and an 8-element pitch or even contiguous planes, see yolo_b200_head.x_row_pitch;
+ * 0 for both 16-bit bits or for a 16-bit bit with FP32X3 or CTA_PAIR) */
 int yolo_b200_head_supported_ex(int c_in, int ny, int nx, int x_row_pitch, int na, int n_classes, int flags);
 /* Candidates exactly as yolo_b200_decode_compact would produce from the head tensor (same record layout, same count /
  * overflow protocol).  Every wait inside the kernel's pipeline is bounded (10 s of wall-clock time without progress):

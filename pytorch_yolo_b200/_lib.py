@@ -47,6 +47,9 @@ VARIANT_BF16 = 0x400
 HEAD_ACCUMULATE = 1
 HEAD_FP32X3 = 8
 HEAD_NO_CANDIDATES = 2
+HEAD_CTA_PAIR = 4
+HEAD_F16 = 0x10
+HEAD_BF16 = 0x20
 
 
 class YoloB200Error(RuntimeError):
@@ -68,6 +71,7 @@ _SIGNATURES = {
     "yolo_b200_compact_from_dense": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int,
                                                C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "yolo_b200_pad_planes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
+    "yolo_b200_pad_planes_16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int, C.c_void_p]),
     "yolo_b200_head_supported": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "yolo_b200_head_supported_ex": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "yolo_b200_head_decode_compact": (C.c_int, [C.POINTER(Head), C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float,

@@ -24,6 +24,16 @@
 // convolution on this GPU with torch's default allow_tf32), so the head values differ from an fp32 CPU convolution by
 // ~1e-3 relative; everything after the accumulator is bit-identical to decode_compact_kernel fed with the head tensor
 // this kernel can also write out (head_out) -- that is the parity test.
+//
+// fp16 / bf16 feature maps (YOLO_B200_HEAD_F16 / _BF16, template parameter DT): the same kernel with a 16-bit main loop.
+// Only the producer, the MMA issuer and the loader warps differ; the epilogue reads the same fp32 accumulators.
+//   X tile  [64 channels] x [128 positions]: two 64-position atoms of 64 x 128-byte rows (8 KB each), plain SWIZZLE_128B
+//           (one 3-D box of 64 x 64 x 2, or a 2-D box of 64 x 64 per atom)                    = A, MN-major
+//   W tile  [NPAD rows] x [64 channels]: one 128-byte row per output channel, SWIZZLE_128B     = B, K-major
+//   tcgen05.mma.cta_group::1.kind::f16 (A and B of the feature map's type, fp32 accumulators), K = 16 per instruction.
+// A stage is 16 KB of X + NPAD x 128 bytes of W: the same 48 KB as the fp32 stage.  Planes without a 16-byte pitch
+// (plane % 8 != 0) but with 4-byte aligned rows (even planes) are filled by the loader warps with 8-byte (plane % 4 == 0)
+// or 4-byte copies; odd planes are padded by the host first (yolo_b200_pad_planes_16).
 #include <cuda.h>          // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 
 #include "common.cuh"
@@ -43,6 +53,10 @@ constexpr int kABytes = 4 * kAtomBytes;    // 16 KB
 constexpr int kMaxN = 256;
 constexpr int kTmemCols = 512;
 constexpr int kWatchdog = 0x100;           // added to *overflow when a pipeline wait times out (never in a correct run)
+// 16-bit main loop: a k-block is 64 channels (one 128-byte W row), an X atom 64 positions x 64 channel rows
+constexpr int kBK16 = 64;
+constexpr int kAtomBytes16 = 64 * kBK16 * 2;     // 8 KB; two atoms = kABytes
+enum : int { kDtF32 = 0, kDtF16 = 1, kDtBF16 = 2 };
 
 struct HeadScale {                         // one detection scale = one head convolution
     alignas(64) CUtensorMap tmap_x;        // [batch*c_in rows][plane] fp32 (row pitch >= plane), box 32 positions x 32 rows
@@ -57,7 +71,8 @@ struct HeadScale {                         // one detection scale = one head con
     int first_tile;                        // first global tile index of this scale (scales are ordered heaviest first)
     int use_x3;                            // tmap_x3 is valid
     int manual;                            // planes without a 16-byte pitch (19x19, 13x13): no tensor map for X, loader warps
-    const float* x;                        // ... fill the stages from here with 4-byte asynchronous copies
+    const float* x;                        // ... fill the stages from here with 4-byte asynchronous copies (16-bit elements
+                                           // with YOLO_B200_HEAD_F16 / _BF16: 8- or 4-byte copies)
     float stride;
     float av[YOLO_B200_MAX_ANCHORS][2];
     float* head_out;                       // optional (batch, NA*(5+NC), ny, nx)
@@ -143,6 +158,12 @@ __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
 __device__ __forceinline__ void cp_async4(uint32_t dst, const float* src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
 }
+__device__ __forceinline__ void cp_async8(uint32_t dst, const void* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
+}
 __device__ __forceinline__ void cp_async_arrive(uint64_t* bar) {
     asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -159,6 +180,14 @@ __device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
         "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"((uint32_t)accumulate) : "memory");
+}
+// D[tmem] (+)= A[smem] * B[smem], fp16 or bf16 inputs (the instruction descriptor says which), fp32 accumulate
+__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, bool accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
         ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"((uint32_t)accumulate) : "memory");
 }
 
@@ -180,6 +209,11 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo_bytes,
 // Instruction descriptor: fp32 accumulator, tf32 A and B, A MN-major (positions contiguous), B K-major, M x N tile.
 __host__ __device__ constexpr uint32_t instr_desc_tf32(int m, int n) {
     return (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (0u << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+// The same for kind::f16: A and B format 0 = F16, 1 = BF16 (fp32 accumulator, A MN-major, B K-major).
+__host__ __device__ constexpr uint32_t instr_desc_f16(int m, int n, bool bf16) {
+    return (1u << 4) | ((bf16 ? 1u : 0u) << 7) | ((bf16 ? 1u : 0u) << 10) | (1u << 15) | (0u << 16) | ((uint32_t)(n >> 3) << 17) |
+           ((uint32_t)(m >> 4) << 24);
 }
 
 // TMEM -> registers: N consecutive columns of this thread's lane (the column may be any offset inside the allocation).
@@ -389,6 +423,17 @@ __device__ __forceinline__ void epilogue_anchor_generic(const HeadParams& P, con
     }
 }
 
+// 16-bit kernel: per ring stage, the producer's hand-over of a loader-filled k-block to the loader warps (one arrival once
+// the stage is free).  The loader warps skip the k-blocks of TMA-filled tiles; waiting on the stage's `empty` barrier after
+// such a skip would compare parities across an unknown number of phases (a CTA whose TMA tiles precede its loader tiles
+// passed the wait early and double-completed the stage's loader barrier).  These barriers complete only for loader-filled
+// k-blocks, in order, and never more than one phase ahead of the loader warps.  Allocated only where it is used.
+template <int S>
+__device__ __forceinline__ uint64_t* xgo_bars() {
+    __shared__ __align__(8) uint64_t bars[S];
+    return bars;
+}
+
 // X3 = fp32-accurate products from three TF32 passes (Markidis-style operand split).  The tensor core truncates an fp32
 // operand to its top 19 bits (sign, exponent, 10 mantissa bits: measured, tests/test_gpu_head.py), so with
 //     x = xhi + xlo,  xhi = trunc_tf32(x),   w = whi + wlo
@@ -402,7 +447,7 @@ __device__ __forceinline__ void epilogue_anchor_generic(const HeadParams& P, con
 constexpr int kConvThreads = 64;           // two auxiliary warps: converters in X3 mode, X loaders for unaligned planes otherwise
 constexpr int kStagesX3 = 2;
 
-template <int NA, int NC, bool WRITE_HEAD, bool LEAKY, bool X3 = false>
+template <int NA, int NC, bool WRITE_HEAD, bool LEAKY, bool X3 = false, int DT = kDtF32>
 __global__ void __launch_bounds__(kProducerThreads + 128 * NA + kConvThreads, 1)
 head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
     // NC == 0: the class count is a run-time value (P.nc) and the accumulator keeps all 256 columns
@@ -410,7 +455,13 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
     constexpr int NPAD = GEN ? kMaxN : (NA * (NC + 5) + 15) / 16 * 16;
     const int NO = GEN ? P.nc + 5 : NC + 5, N = NA * NO;
     static_assert(NPAD <= kMaxN, "one accumulator stage holds at most 256 output channels");
-    constexpr int kBBytes = NPAD * kBK * 4;
+    // 16-bit feature maps: the k-block, the X atom and the MMA's K differ; the stage sizes are those of fp32
+    constexpr bool H = DT != kDtF32;
+    static_assert(!(H && X3), "the three-pass mode is fp32 only");
+    constexpr int BK = H ? kBK16 : kBK;            // channels per stage
+    constexpr int AS = H ? 6 : 5, AP = 1 << AS;   // positions per X swizzle atom, and its log2
+    constexpr int kAtom = H ? kAtomBytes16 : kAtomBytes;
+    constexpr int kBBytes = NPAD * kBK * 4;        // = NPAD * kBK16 * 2
     constexpr int kStages = X3 ? kStagesX3 : hd::kStages;
     constexpr int kXBytes = X3 ? 2 * kABytes : kABytes;           // X (and its low part)
     constexpr int kStageBytes = kXBytes + (X3 ? 2 : 1) * kBBytes;
@@ -439,6 +490,10 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
         for (int s = 0; s < kStages; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); mbar_init(&conv[s], X3 ? kConvThreads / 32 : kConvThreads); }
 #pragma unroll
         for (int s = 0; s < 2; ++s) { mbar_init(&tfull[s], 1); mbar_init(&tempty[s], 4 * NA); }
+        if constexpr (H) {
+#pragma unroll
+            for (int s = 0; s < kStages; ++s) mbar_init(&xgo_bars<kStages>()[s], 1);
+        }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -478,11 +533,12 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                 int k, img, p0, np;
                 locate(tile, k, img, p0, np);
                 const HeadScale& S = P.sc[k];
-                const int atoms = (np + 31) >> 5;             // boxes that start inside the plane; the rest stays stale
+                const int atoms = (np + AP - 1) >> AS;         // boxes that start inside the plane; the rest stays stale
                 // One 3-D box brings all four atoms of a k-block (a TMA instruction costs the producer ~70 ns whatever its
                 // size -- profiles/r01_l_*: four boxes per k-block made the issue rate the bound).  The 3-D view only holds
                 // the plane's complete 32-position atoms, so the tile with the ragged last atom uses 2-D boxes.
-                const bool one_box = S.use_x3 && (np & 31) == 0;
+                // (16-bit: two atoms of 64 positions, the same rules.)
+                const bool one_box = S.use_x3 && (np & (AP - 1)) == 0;
                 for (int kb = 0; kb < S.kblocks; ++kb, ++it) {
                     const int st = (int)(it % kStages);
                     mbar_wait(&empty[st], ((it / kStages) & 1u) ^ 1u, P.overflow, 1);
@@ -490,17 +546,20 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                     // profiling modes (bits 1, 2 of skip_epilogue): fetch W / X only during the first trip round the ring
                     const bool load_w = !(P.skip_epilogue & 2) || it < (uint32_t)kStages;
                     const bool load_x = (!(P.skip_epilogue & 4) || it < (uint32_t)kStages) && !S.manual;   // manual: the loader warps
-                    mbar_expect_tx(&full[st], (uint32_t)((load_x ? (one_box ? kABytes : atoms * kAtomBytes) : 0) +
+                    mbar_expect_tx(&full[st], (uint32_t)((load_x ? (one_box ? kABytes : atoms * kAtom) : 0) +
                                                          (load_w ? (X3 ? 2 : 1) * kBBytes : 0)));
                     if (load_x) {
                         if (one_box)
-                            tma_tile3_g2s(a_s, &S.tmap_x3, 0, img * S.c_in + kb * kBK, p0 >> 5, &full[st]);
+                            tma_tile3_g2s(a_s, &S.tmap_x3, 0, img * S.c_in + kb * BK, p0 >> AS, &full[st]);
                         else
                             for (int j = 0; j < atoms; ++j)
-                                tma_tile_g2s(a_s + (uint32_t)j * kAtomBytes, &S.tmap_x, p0 + 32 * j, img * S.c_in + kb * kBK, &full[st]);
+                                tma_tile_g2s(a_s + (uint32_t)j * kAtom, &S.tmap_x, p0 + AP * j, img * S.c_in + kb * BK, &full[st]);
+                    }
+                    if constexpr (H) {
+                        if (S.manual) mbar_arrive(&xgo_bars<kStages>()[st]);   // the loader warps may fill this stage
                     }
                     if (load_w) {
-                        tma_tile_g2s(a_s + kXBytes, &S.tmap_w, kb * kBK, 0, &full[st]);
+                        tma_tile_g2s(a_s + kXBytes, &S.tmap_w, kb * BK, 0, &full[st]);
                         if constexpr (X3) tma_tile_g2s(a_s + kXBytes + kBBytes, &S.tmap_w, kb * kBK, kMaxN, &full[st]);   // rows 256..: w - trunc(w)
                     }
                 }
@@ -509,7 +568,7 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
     } else if (warp == 1) {
         // ===== MMA issuer =====
         if (lane == 0) {
-            constexpr uint32_t idesc = instr_desc_tf32(kM, NPAD);
+            constexpr uint32_t idesc = H ? instr_desc_f16(kM, NPAD, DT == kDtBF16) : instr_desc_tf32(kM, NPAD);
             uint32_t it = 0, xparity = 0;
             int tl = 0;
             for (int tile = blockIdx.x; tile < P.n_tiles; tile += gridDim.x, ++tl) {
@@ -533,6 +592,18 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                     tc_fence_after();
                     if (P.skip_epilogue & 8) { mbar_arrive(&empty[st]); continue; }   // profiling: the stream without the tensor core
                     const uint32_t a_s = ring + (uint32_t)st * kStageBytes, b_s = a_s + kXBytes;
+                    if constexpr (H) {
+#pragma unroll
+                        for (int kk = 0; kk < kBK16 / 16; ++kk) {
+                            // A: MN-major SWIZZLE_128B: an atom is 64 positions (one 128-byte row per channel) x 8 channels;
+                            //    the tile's two 64-position atoms are kAtomBytes16 apart (LBO), 8-channel groups 1 KB apart
+                            //    (SBO), so this instruction's 16 channels start 2 KB after the previous one's
+                            // B: K-major, as in fp32: 8-row groups 1 KB apart (SBO); 16 channels = 32 bytes inside the row
+                            const uint64_t ad = smem_desc(a_s + (uint32_t)kk * 2048u, kAtomBytes16, 1024u, kSw128);
+                            const uint64_t bd = smem_desc(b_s + (uint32_t)kk * 32u, 16u, 1024u, kSw128);
+                            umma_f16(d_tmem, ad, bd, idesc, (kb | kk) != 0);
+                        }
+                    } else {
 #pragma unroll
                     for (int kk = 0; kk < kBK / 8; ++kk) {
                         // A: MN-major, 32-byte-base swizzle: 4 atoms of 32 positions kAtomBytes apart (LBO); one channel is one
@@ -549,6 +620,7 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                             umma_tf32(d_tmem, ad_lo, bd, idesc, true);
                         }
                     }
+                    }
                     umma_commit(&empty[st]);          // the stage is free once these MMAs have read it
                 }
                 if (P.skip_epilogue & 8) mbar_arrive(&tfull[acc]);
@@ -564,11 +636,47 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
         // 32-byte chunk (position / 8) % 4 XOR-ed with r % 4.  Lanes run along positions: coalesced 128-byte reads.
         const int lt = (int)threadIdx.x - (kProducerThreads + 128 * NA);
         uint32_t it = 0;
+        uint32_t gparity = 0;                         // 16-bit: phase parity of each stage's hand-over barrier
         for (int tile = blockIdx.x; tile < P.n_tiles; tile += gridDim.x) {
             int k, img, p0, np;
             locate(tile, k, img, p0, np);
             const HeadScale& S = P.sc[k];
             if (!S.manual) { it += (uint32_t)S.kblocks; continue; }
+            if constexpr (H) {
+                // 16-bit (planes with 4-byte aligned rows, plane % 8 != 0): TMA's SWIZZLE_128B layout -- atom = position / 64
+                // (8 KB), channel row r at r * 128 bytes, the 16-byte chunk (position / 8) % 8 XOR-ed with r % 8.
+                //   plane % 4 == 0: 8-byte copies of 4 positions; lane = 4-position group (256 contiguous bytes per warp and
+                //                   row), warp w of the two takes channel rows 32 w .. 32 w + 31 of every k-block;
+                //   plane % 4 == 2: 4-byte copies of 2 positions; a thread owns positions 2 lt, 2 lt + 1 in all 64 rows.
+                // The row-dependent parts of the offset are compile-time after unrolling (r % 8 == i % 8).
+                const uint16_t* tile_src = reinterpret_cast<const uint16_t*>(S.x) + (size_t)img * S.c_in * S.plane + p0;
+                const bool wide = (S.plane & 3) == 0;
+                const int p = wide ? 4 * (lt & 31) : 2 * lt;
+                const int r0 = wide ? 32 * (lt >> 5) : 0;
+                const bool v = p < np;
+                const uint32_t d = (uint32_t)((p >> 6) * kAtomBytes16 + (p & 7) * 2 + r0 * 128);
+                const int c = (p >> 3) & 7;
+                uint32_t xo[8];
+#pragma unroll
+                for (int q = 0; q < 8; ++q) xo[q] = d + (uint32_t)((c ^ q) << 4);
+                for (int kb = 0; kb < S.kblocks; ++kb, ++it) {
+                    const int st = (int)(it % kStages);
+                    mbar_wait(&xgo_bars<kStages>()[st], (gparity >> st) & 1u, P.overflow, 7);   // the stage is free
+                    gparity ^= 1u << st;
+                    const uint32_t a_s = ring + (uint32_t)st * kStageBytes;
+                    const uint16_t* src = tile_src + (size_t)(kb * kBK16 + r0) * S.plane + p;
+                    if (v) {
+                        if (wide) {
+#pragma unroll
+                            for (int i = 0; i < 32; ++i, src += S.plane) cp_async8(a_s + (uint32_t)(i * 128) + xo[i & 7], src);
+                        } else {
+#pragma unroll
+                            for (int i = 0; i < kBK16; ++i, src += S.plane) cp_async4(a_s + (uint32_t)(i * 128) + xo[i & 7], src);
+                        }
+                    }
+                    cp_async_arrive(&conv[st]);
+                }
+            } else {
             // a thread owns two positions of the tile, lt and lt + 64, for all 32 channel rows of every k-block: the
             // position-dependent parts of the shared-memory offset are computed once per tile, the row-dependent ones are
             // compile-time after unrolling, and the source pointers advance by one plane per row
@@ -591,6 +699,7 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                     if (vb) cp_async4(a_s + (uint32_t)(r * 128) + xb_[r & 3], src + pb);
                 }
                 cp_async_arrive(&conv[st]);
+            }
             }
         }
     } else if (X3 && warp >= 2 + 4 * NA) {
@@ -888,6 +997,32 @@ pad_planes_kernel(const float* __restrict__ x, float* __restrict__ out, long lon
         }
     }
 }
+
+// The same for 2-byte elements (fp16 / bf16 feature maps), pitch % 8 == 0: gives planes of any size -- odd ones above all,
+// whose rows the kernel's loader warps cannot copy in aligned pieces -- the 16-byte row pitch TMA needs.
+__global__ void __launch_bounds__(kPadThreads)
+pad_planes16_kernel(const uint16_t* __restrict__ x, uint16_t* __restrict__ out, long long rows, int plane, int pitch) {
+    const int lane = threadIdx.x & 31;
+    const long long warp0 = (long long)blockIdx.x * (kPadThreads / 32) + (threadIdx.x >> 5);
+    const long long stride = (long long)gridDim.x * (kPadThreads / 32);
+    for (long long r = warp0; r < rows; r += stride) {
+        const uint16_t* src = x + r * plane;
+        uint16_t* dst = out + r * pitch;
+        for (int base = 0; base < pitch; base += 32 * kPadMaxIter) {
+            unsigned short v[kPadMaxIter];
+#pragma unroll
+            for (int k = 0; k < kPadMaxIter; ++k) {
+                const int i = base + 32 * k + lane;
+                v[k] = i < plane ? ldg_stream_b16(src + i) : (unsigned short)0;
+            }
+#pragma unroll
+            for (int k = 0; k < kPadMaxIter; ++k) {
+                const int i = base + 32 * k + lane;
+                if (i < pitch) dst[i] = v[k];
+            }
+        }
+    }
+}
 }  // namespace hd
 }  // namespace yb
 
@@ -909,18 +1044,33 @@ extern "C" int yolo_b200_pad_planes(const float* x, float* out, long long rows, 
     return (int)cudaGetLastError();
 }
 
+extern "C" int yolo_b200_pad_planes_16(const void* x, void* out, long long rows, int plane, int pitch, yolo_b200_stream_t stream) {
+    if (rows > 0 && (!x || !out)) return YOLO_B200_E_NULL;
+    if (rows < 0 || plane < 1 || pitch < plane || pitch % 8 != 0) return YOLO_B200_E_RANGE;
+    if (((uintptr_t)x & 1u) || ((uintptr_t)out & 15u)) return YOLO_B200_E_ALIGN;
+    if (rows == 0) return 0;
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const long long want = (rows + hd::kPadThreads / 32 - 1) / (hd::kPadThreads / 32);
+    const int grid = (int)(want < (long long)sms * 8 ? want : (long long)sms * 8);
+    hd::pad_planes16_kernel<<<grid, hd::kPadThreads, 0, stream>>>(static_cast<const uint16_t*>(x), static_cast<uint16_t*>(out), rows,
+                                                                  plane, pitch);
+    return (int)cudaGetLastError();
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 static int encode_2d(EncodeTiledFn fn, CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer, uint64_t row_bytes,
                      uint32_t box_inner, uint32_t box_outer, CUtensorMapSwizzle swizzle,
-                     CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B) {
+                     CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_FLOAT32) {
     const cuuint64_t gdim[2] = {inner, outer};
     const cuuint64_t gstride[1] = {row_bytes};
     const cuuint32_t box[2] = {box_inner, box_outer};
     const cuuint32_t estr[2] = {1, 1};
-    const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), gdim, gstride, box, estr,
+    const CUresult r = fn(map, dtype, 2, const_cast<void*>(base), gdim, gstride, box, estr,
                           CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, promo,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? 0 : YOLO_B200_E_RANGE;
@@ -929,8 +1079,16 @@ static int encode_2d(EncodeTiledFn fn, CUtensorMap* map, const void* base, uint6
 typedef void (*HeadKernel)(const hd::HeadParams);
 
 // the (anchors per scale, classes) pairs the epilogue is instantiated for, each with / without head_out stores and LeakyReLU
+template <int NA, int NC, int DT>
+static HeadKernel pick_variant16(bool write_head, bool leaky) {
+    return write_head ? (leaky ? hd::head_decode_compact_kernel<NA, NC, true, true, false, DT> : hd::head_decode_compact_kernel<NA, NC, true, false, false, DT>)
+                      : (leaky ? hd::head_decode_compact_kernel<NA, NC, false, true, false, DT> : hd::head_decode_compact_kernel<NA, NC, false, false, false, DT>);
+}
 template <int NA, int NC>
-static HeadKernel pick_variant(bool write_head, bool leaky, bool pair, bool x3 = false) {
+static HeadKernel pick_variant(bool write_head, bool leaky, bool pair, bool x3 = false, int dt = hd::kDtF32) {
+    // 16-bit feature maps: the one-pass single-CTA kernel only
+    if (dt == hd::kDtF16) return pair || x3 ? nullptr : pick_variant16<NA, NC, hd::kDtF16>(write_head, leaky);
+    if (dt == hd::kDtBF16) return pair || x3 ? nullptr : pick_variant16<NA, NC, hd::kDtBF16>(write_head, leaky);
     if (x3) {
         if constexpr (NC == 80 || NC == 0) {
             return write_head ? (leaky ? hd::head_decode_compact_kernel<NA, NC, true, true, true> : hd::head_decode_compact_kernel<NA, NC, true, false, true>)
@@ -950,16 +1108,16 @@ static HeadKernel pick_variant(bool write_head, bool leaky, bool pair, bool x3 =
     return write_head ? (leaky ? hd::head_decode_compact_kernel<NA, NC, true, true> : hd::head_decode_compact_kernel<NA, NC, true, false>)
                       : (leaky ? hd::head_decode_compact_kernel<NA, NC, false, true> : hd::head_decode_compact_kernel<NA, NC, false, false>);
 }
-static HeadKernel head_kernel_for(int na, int nc, bool write_head, bool leaky, bool pair, bool x3 = false) {
+static HeadKernel head_kernel_for(int na, int nc, bool write_head, bool leaky, bool pair, bool x3 = false, int dt = hd::kDtF32) {
     if (x3) {     // three-pass mode: the 80-class epilogue or the run-time class loop, both over all 256 accumulator columns
         if (na == 3 && nc == 80) return pick_variant<3, 80>(write_head, leaky, false, true);
         if (na == 3 && nc >= 1 && na * (nc + 5) <= hd::kMaxN) return pick_variant<3, 0>(write_head, leaky, false, true);
         return nullptr;
     }
-    if (na == 3 && nc == 80) return pick_variant<3, 80>(write_head, leaky, pair);     // COCO
-    if (na == 3 && nc == 20) return pick_variant<3, 20>(write_head, leaky, pair);     // VOC
-    if (na == 3 && nc == 1) return pick_variant<3, 1>(write_head, leaky, pair);
-    if (na == 3 && nc >= 2 && na * (nc + 5) <= hd::kMaxN && !pair) return pick_variant<3, 0>(write_head, leaky, false);   // any other class count
+    if (na == 3 && nc == 80) return pick_variant<3, 80>(write_head, leaky, pair, false, dt);     // COCO
+    if (na == 3 && nc == 20) return pick_variant<3, 20>(write_head, leaky, pair, false, dt);     // VOC
+    if (na == 3 && nc == 1) return pick_variant<3, 1>(write_head, leaky, pair, false, dt);
+    if (na == 3 && nc >= 2 && na * (nc + 5) <= hd::kMaxN && !pair) return pick_variant<3, 0>(write_head, leaky, false, false, dt);   // any other class count
     return nullptr;
 }
 // output-channel rows the kernel's accumulator / W tile holds for (na, nc)
@@ -968,7 +1126,24 @@ static int head_npad(int na, int nc) {
     return specialised ? (na * (nc + 5) + 15) / 16 * 16 : hd::kMaxN;
 }
 
+// element type of X and W named by the flags: fp32, fp16, bf16, or -1 for both 16-bit bits
+static int head_dtype(int flags) {
+    const int h = flags & (YOLO_B200_HEAD_F16 | YOLO_B200_HEAD_BF16);
+    return h == 0 ? hd::kDtF32 : h == YOLO_B200_HEAD_F16 ? hd::kDtF16 : h == YOLO_B200_HEAD_BF16 ? hd::kDtBF16 : -1;
+}
+
 extern "C" int yolo_b200_head_supported_ex(int c_in, int ny, int nx, int x_row_pitch, int na, int n_classes, int flags) {
+    const int dt = head_dtype(flags);
+    if (dt != hd::kDtF32) {
+        // 16-bit: one-pass single-CTA kernel, 64-channel k-blocks, a row pitch of 8 elements (16 bytes) unless the
+        // contiguous planes are even (the loader warps copy 4-byte aligned pieces; odd planes go through the padded copy)
+        if (dt < 0 || (flags & (YOLO_B200_HEAD_FP32X3 | YOLO_B200_HEAD_CTA_PAIR))) return 0;
+        if (c_in < hd::kBK16 || c_in % hd::kBK16 != 0 || ny < 1 || nx < 1) return 0;
+        const long long plane = (long long)ny * nx, pitch = x_row_pitch ? x_row_pitch : plane;
+        if (pitch < plane) return 0;
+        if (pitch % 8 != 0 && (x_row_pitch != 0 || plane % 2 != 0)) return 0;
+        return head_kernel_for(na, n_classes, false, false, false, false, dt) != nullptr ? 1 : 0;
+    }
     if (c_in < hd::kBK || c_in % hd::kBK != 0) return 0;
     if (ny < 1 || nx < 1) return 0;
     const long long pitch = x_row_pitch ? x_row_pitch : (long long)ny * nx;
@@ -992,6 +1167,10 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
     const bool emit = (flags & YOLO_B200_HEAD_NO_CANDIDATES) == 0;
     const bool x3 = (flags & YOLO_B200_HEAD_FP32X3) != 0;
     if (x3 && (flags & YOLO_B200_HEAD_CTA_PAIR)) return YOLO_B200_E_RANGE;
+    const int dt = head_dtype(flags);
+    if (dt < 0) return YOLO_B200_E_RANGE;
+    const bool h16 = dt != hd::kDtF32;
+    if (h16 && (flags & (YOLO_B200_HEAD_FP32X3 | YOLO_B200_HEAD_CTA_PAIR))) return YOLO_B200_E_UNSUPPORTED;
     if (emit && (!cand_box || !cand_meta)) return YOLO_B200_E_NULL;
     if (n_heads < 1 || n_heads > YOLO_B200_MAX_SCALES || batch < 0 || nc < 1 || rows_per_img < 1 || (emit && cap_per_img < 1))
         return YOLO_B200_E_RANGE;
@@ -1030,7 +1209,12 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
 
     // L2 promotion 64 B .. 256 B and the plain 128-byte swizzle make no measurable difference for the X stream
     // (profiles/r01_l_tma_box_rows_experiment.txt); MN-major tf32 requires the 32-byte-atom swizzle.
-    const CUtensorMapSwizzle x_swizzle = CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
+    // 16-bit: plain SWIZZLE_128B, the MN-major layout kind::f16 reads; 64-position atoms
+    const CUtensorMapSwizzle x_swizzle = h16 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
+    const CUtensorMapDataType x_type = dt == hd::kDtF16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16
+                                      : dt == hd::kDtBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    const uint64_t esz = h16 ? 2 : 4;
+    const int bk = h16 ? hd::kBK16 : hd::kBK, ap = h16 ? 64 : 32;
     const CUtensorMapL2promotion x_promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
     const int no = nc + 5;
 
@@ -1053,34 +1237,35 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
             const yolo_b200_head& h = heads[order[i]];
             hd::HeadScale& S = P.sc[i];
             const int plane = h.scale.ny * h.scale.nx;
-            const uint64_t pitch = h.x_row_pitch ? (uint64_t)h.x_row_pitch : (uint64_t)plane;      // floats between channel planes
+            const uint64_t pitch = h.x_row_pitch ? (uint64_t)h.x_row_pitch : (uint64_t)plane;      // elements between channel planes
             int rc;
-            S.manual = pitch % 4 != 0 ? 1 : 0;        // (validated above: contiguous planes, one-pass single-CTA kernel)
+            S.manual = pitch % (16 / esz) != 0 ? 1 : 0;   // (validated above: contiguous planes, one-pass single-CTA kernel)
             S.x = h.x;
             if (!S.manual &&
-                (rc = encode_2d(encode, &S.tmap_x, h.x, (uint64_t)plane, (uint64_t)batch * h.c_in, pitch * 4, 32, hd::kBK, x_swizzle, x_promo)))
+                (rc = encode_2d(encode, &S.tmap_x, h.x, (uint64_t)plane, (uint64_t)batch * h.c_in, pitch * esz, ap, bk, x_swizzle, x_promo, x_type)))
                 return rc;
             // (three-pass mode: the tensor holds 512 rows, the low parts of the weights behind the weights)
-            if ((rc = encode_2d(encode, &S.tmap_w, h.weight, (uint64_t)h.c_in, (uint64_t)(x3 ? 2 * npad : npad), (uint64_t)h.c_in * 4, hd::kBK,
-                                (uint32_t)npad, CU_TENSOR_MAP_SWIZZLE_128B)))
+            if ((rc = encode_2d(encode, &S.tmap_w, h.weight, (uint64_t)h.c_in, (uint64_t)(x3 ? 2 * npad : npad), (uint64_t)h.c_in * esz, bk,
+                                (uint32_t)npad, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, x_type)))
                 return rc;
-            if ((rc = encode_2d(encode, &S.tmap_w2, h.weight, (uint64_t)h.c_in, (uint64_t)npad, (uint64_t)h.c_in * 4, hd::kBK, (uint32_t)npad / 2,
-                                CU_TENSOR_MAP_SWIZZLE_128B)))
+            if (!h16 && (rc = encode_2d(encode, &S.tmap_w2, h.weight, (uint64_t)h.c_in, (uint64_t)npad, (uint64_t)h.c_in * 4, hd::kBK,
+                                        (uint32_t)npad / 2, CU_TENSOR_MAP_SWIZZLE_128B)))
                 return rc;
-            // 3-D view over the complete 32-position atoms of every row; rows are pitch*4 bytes apart, atoms 128 bytes
+            // 3-D view over the complete atoms (32 positions, 16-bit: 64) of every row; rows are pitch elements apart, atoms
+            // 128 bytes; the box is the tile's four (16-bit: two) atoms
             S.use_x3 = 0;
-            if (plane >= 32 && !S.manual) {
-                const cuuint64_t gdim[3] = {32, (cuuint64_t)batch * h.c_in, (cuuint64_t)(plane / 32)};
-                const cuuint64_t gstride[2] = {(cuuint64_t)pitch * 4, 128};
-                const cuuint32_t box[3] = {32, (cuuint32_t)hd::kBK, 4};
+            if (plane >= ap && !S.manual) {
+                const cuuint64_t gdim[3] = {(cuuint64_t)ap, (cuuint64_t)batch * h.c_in, (cuuint64_t)(plane / ap)};
+                const cuuint64_t gstride[2] = {(cuuint64_t)pitch * esz, 128};
+                const cuuint32_t box[3] = {(cuuint32_t)ap, (cuuint32_t)bk, (cuuint32_t)(hd::kM / ap)};
                 const cuuint32_t estr[3] = {1, 1, 1};
-                const CUresult r3 = encode(&S.tmap_x3, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(h.x), gdim, gstride, box, estr,
+                const CUresult r3 = encode(&S.tmap_x3, x_type, 3, const_cast<float*>(h.x), gdim, gstride, box, estr,
                                            CU_TENSOR_MAP_INTERLEAVE_NONE, x_swizzle, x_promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
                 S.use_x3 = r3 == CUDA_SUCCESS ? 1 : 0;        // a driver that rejects the view leaves the 2-D boxes
             }
             for (int o = 0; o < hd::kMaxN; ++o) S.bias[o] = o < n ? h.bias_host[o] : 0.0f;
             S.slope = h.negative_slope;
-            S.c_in = h.c_in; S.kblocks = h.c_in / hd::kBK;
+            S.c_in = h.c_in; S.kblocks = h.c_in / bk;
             S.ny = h.scale.ny; S.nx = h.scale.nx; S.plane = plane; S.row_off = h.scale.row_off;
             S.tiles_per_img = (plane + hd::kM - 1) / hd::kM;
             S.first_tile = (int)tiles;
@@ -1117,7 +1302,7 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
             }
             continue;
         }
-        HeadKernel kern = head_kernel_for(na, nc, write_head, leaky, false, x3);
+        HeadKernel kern = head_kernel_for(na, nc, write_head, leaky, false, x3, dt);
         if (!kern) return YOLO_B200_E_UNSUPPORTED;
         const size_t smem = x3 ? (size_t)hd::kStagesX3 * 2 * (hd::kABytes + (size_t)npad * hd::kBK * 4) + 1024
                                : (size_t)hd::kStages * (hd::kABytes + (size_t)npad * hd::kBK * 4) + 1024;

@@ -22,6 +22,8 @@ MAX_PER_CLASS = 100    # reference utils/utils.py:247-250
 _FP32 = (torch.float32,)
 # head dtypes decode_compact reads, and the variant bit that tells the library (include/yolo_b200.h)
 HEAD_DTYPE_BITS = {torch.float32: 0, torch.float16: _lib.VARIANT_F16, torch.bfloat16: _lib.VARIANT_BF16}
+# feature-map dtypes the fused head kernel reads, and the flag that tells the library
+FEATURE_DTYPE_FLAGS = {torch.float32: 0, torch.float16: _lib.HEAD_F16, torch.bfloat16: _lib.HEAD_BF16}
 
 
 def _require_cuda(t: torch.Tensor, what: str) -> None:
@@ -220,7 +222,8 @@ def decode_compact(heads, specs, nc: int, conf_thres: float, buf: Buffers, min_w
 @dataclass
 class HeadWeights:
     """A head convolution folded for the fused kernel (what ConvBlock.fuse computes, reference
-    models/yolo_base.py:46-57): ``weight`` (256, c_in) on the device with pad rows zero, ``bias`` on the host."""
+    models/yolo_base.py:46-57): ``weight`` (256, c_in) on the device with pad rows zero, ``bias`` on the host.
+    ``weight.dtype`` is the kernel's operand type: the feature maps must have the same one."""
 
     weight: torch.Tensor
     bias: torch.Tensor             # (n_out,) fp32 CPU
@@ -231,6 +234,10 @@ class HeadWeights:
     @property
     def c_in(self) -> int:
         return self.weight.shape[1]
+
+    @property
+    def dtype(self) -> torch.dtype:
+        return self.weight.dtype
 
     def bias_array(self):
         """The bias as the ``const float*`` host array the C ABI takes (built once)."""
@@ -245,11 +252,17 @@ def tf32_trunc(t: torch.Tensor) -> torch.Tensor:
     return (t.contiguous().view(torch.int32) & -8192).view(torch.float32)
 
 
-def fold_head(module: torch.nn.Module, device=None, fp32x3: bool = False) -> HeadWeights:
+def fold_head(module: torch.nn.Module, device=None, fp32x3: bool = False, dtype: torch.dtype = torch.float32) -> HeadWeights:
     """Fold a reference head -- ``ConvBlock(c_in, na*(5+nc), size=1)`` = Conv2d(bias=False) + BatchNorm2d + LeakyReLU(0.1)
     (models/yolov3_spp.py:86,99,111) or a plain ``nn.Conv2d(c_in, na*(5+nc), 1)`` (models/yolov3_tiny.py:38,42) -- into one
     (256, c_in) weight matrix (rows beyond the head's channels zero), one bias vector and an activation slope.
-    BatchNorm uses its running statistics (eval mode)."""
+    BatchNorm uses its running statistics (eval mode).
+    ``dtype``: the kernel's operand type, float32 or (for fp16 / bf16 feature maps) float16 / bfloat16.  The fold runs in
+    fp64 and is rounded to fp32, then to ``dtype``: those are the operands the tensor core multiplies.  The bias stays fp32."""
+    if dtype not in FEATURE_DTYPE_FLAGS:
+        raise TypeError(f"fold_head: dtype must be float32, float16 or bfloat16, got {dtype}")
+    if fp32x3 and dtype != torch.float32:
+        raise ValueError("fp32x3 splits fp32 operands: it cannot be combined with a 16-bit dtype")
     leaves = [m for m in module.modules() if isinstance(m, (torch.nn.Conv2d, torch.nn.BatchNorm2d, torch.nn.LeakyReLU))]
     convs = [m for m in leaves if isinstance(m, torch.nn.Conv2d)]
     bns = [m for m in leaves if isinstance(m, torch.nn.BatchNorm2d)]
@@ -274,37 +287,51 @@ def fold_head(module: torch.nn.Module, device=None, fp32x3: bool = False) -> Hea
     wp[:n_out] = w.float()
     if fp32x3:                                                           # rows 256..: w - trunc_tf32(w), exact in fp32
         wp[256:256 + n_out] = wp[:n_out] - tf32_trunc(wp[:n_out])
+    if dtype != torch.float32:
+        w16 = wp.to(dtype)
+        if bool(torch.isfinite(wp).all()) and not bool(torch.isfinite(w16).all()):
+            raise ValueError(f"folded head weights reach {float(wp.abs().max()):.6g}, beyond the {dtype} range")
+        wp = w16
     dev = device if device is not None else conv.weight.device
     return HeadWeights(wp.to(dev).contiguous(), b.float().contiguous(), float(acts[0].negative_slope) if acts else 1.0, n_out,
                        fp32x3)
 
 
-def head_supported(c_in: int, spec: ScaleSpec, nc: int, row_pitch: int = 0, fp32x3: bool = False) -> bool:
+def head_supported(c_in: int, spec: ScaleSpec, nc: int, row_pitch: int = 0, fp32x3: bool = False,
+                   dtype: torch.dtype = torch.float32) -> bool:
     """Does the tensor-core kernel take this scale?  Contiguous planes that are not a multiple of 4 floats (19x19, 13x13) are
-    read in place by the one-pass kernel; the three-pass mode needs them padded (``row_pitch = padded_pitch(spec)``)."""
-    return bool(_lib.load().yolo_b200_head_supported_ex(c_in, spec.ny, spec.nx, row_pitch, spec.na, nc,
-                                                        _lib.HEAD_FP32X3 if fp32x3 else 0))
+    read in place by the one-pass kernel; the three-pass mode needs them padded (``row_pitch = padded_pitch(spec)``).
+    ``dtype`` float16 / bfloat16: feature maps of that type (c_in a multiple of 64; planes that are not a multiple of 8
+    elements are read in place when even, odd ones need ``row_pitch = padded_pitch(spec, dtype)``)."""
+    flags = (_lib.HEAD_FP32X3 if fp32x3 else 0) | FEATURE_DTYPE_FLAGS[dtype]
+    return bool(_lib.load().yolo_b200_head_supported_ex(c_in, spec.ny, spec.nx, row_pitch, spec.na, nc, flags))
 
 
-def padded_pitch(spec: ScaleSpec) -> int:
-    """Floats per channel plane after padding to the 16-byte TMA row pitch (361 -> 364, 169 -> 172)."""
-    return (spec.ny * spec.nx + 3) // 4 * 4
+def padded_pitch(spec: ScaleSpec, dtype: torch.dtype = torch.float32) -> int:
+    """Elements per channel plane after padding to the 16-byte TMA row pitch: a multiple of 4 floats (361 -> 364,
+    169 -> 172) or of 8 fp16 / bf16 elements (361 -> 368, 169 -> 176)."""
+    q = 4 if dtype == torch.float32 else 8
+    return (spec.ny * spec.nx + q - 1) // q * q
 
 
 def pad_feature(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """(B, C, ny, nx) -> (B, C, pitch) with every channel plane padded to a multiple of 4 floats: the form in which the
-    fused head kernel accepts feature maps whose plane is not (19x19, 13x13).  One read and one write of the map."""
-    _require_cuda(x, "feature map")
+    """(B, C, ny, nx) -> (B, C, pitch) with every channel plane padded to a 16-byte row pitch (a multiple of 4 floats, or
+    of 8 fp16 / bf16 elements): the form in which the fused head kernel accepts feature maps whose plane is not (19x19,
+    13x13).  One read and one write of the map.  ``out``, if given, has the feature map's dtype."""
+    _require_device(x, "feature map")
+    _require_dtype(x, "feature map", tuple(FEATURE_DTYPE_FLAGS))
     b, c, ny, nx = x.shape
-    pitch = (ny * nx + 3) // 4 * 4
+    q = 4 if x.dtype == torch.float32 else 8
+    pitch = (ny * nx + q - 1) // q * q
     if out is None:
         out = torch.empty(b, c, pitch, dtype=x.dtype, device=x.device)
-    elif out.shape != (b, c, pitch) or not out.is_contiguous() or out.device != x.device or out.dtype != torch.float32:
-        raise ValueError(f"out must be a contiguous fp32 (B, C, {pitch}) tensor on the feature map's device")
+    elif out.shape != (b, c, pitch) or not out.is_contiguous() or out.device != x.device or out.dtype != x.dtype:
+        raise ValueError(f"out must be a contiguous {x.dtype} (B, C, {pitch}) tensor on the feature map's device")
     x = x if x.is_contiguous() else x.contiguous()
+    lib = _lib.load()
+    fn = lib.yolo_b200_pad_planes if x.dtype == torch.float32 else lib.yolo_b200_pad_planes_16
     with torch.cuda.device(x.device):
-        check(_lib.load().yolo_b200_pad_planes(x.data_ptr(), out.data_ptr(), b * c, ny * nx, pitch, _stream_ptr(x.device)),
-              "yolo_b200_pad_planes")
+        check(fn(x.data_ptr(), out.data_ptr(), b * c, ny * nx, pitch, _stream_ptr(x.device)), "yolo_b200_pad_planes")
     return out
 
 
@@ -315,7 +342,8 @@ def head_decode_compact(feats: Sequence[torch.Tensor], weights: Sequence[HeadWei
                         _profile_flags: int = 0, cta_pair: bool = False) -> None:
     """1x1 head convolution (+ folded BatchNorm + LeakyReLU) on the tensor cores, decoded and compacted straight from the
     accumulator into ``buf``.  ``feats[k]``: (B, c_in, ny, nx) input of head k; ``row_offs[k]``: first row of scale k in the
-    concatenated prediction.  ``head_outs[k]`` (optional) receives the activated head tensor (B, na*(5+nc), ny, nx).
+    concatenated prediction.  The feature maps are float32, float16 or bfloat16, one dtype for all and the one the weights
+    were folded to (``fold_head(..., dtype=)``).  ``head_outs[k]`` (optional) receives the activated head tensor (B, na*(5+nc), ny, nx).
     ``cta_pair`` selects the tcgen05 ``cta_group::2`` variant of the kernel (identical results)."""
     lib = _lib.load()
     n = len(feats)
@@ -326,7 +354,14 @@ def head_decode_compact(feats: Sequence[torch.Tensor], weights: Sequence[HeadWei
     dev = feats[0].device
     batch = feats[0].shape[0]
     for k, (x, hw, sp) in enumerate(zip(feats, weights, specs)):
-        _require_cuda(x, f"feature map {k}")
+        _require_device(x, f"feature map {k}")
+        _require_dtype(x, f"feature map {k}", tuple(FEATURE_DTYPE_FLAGS))
+        if x.dtype != feats[0].dtype:
+            raise ValueError(f"all feature maps of one call must share a dtype: feature map 0 is {feats[0].dtype}, "
+                             f"feature map {k} {x.dtype}")
+        if hw.dtype != x.dtype:
+            raise ValueError(f"feature map {k} is {x.dtype} but its head weights are folded to {hw.dtype} "
+                             "(ops.fold_head(..., dtype=))")
         pitch = 0
         if x.dim() == 3 and x.shape[0] == batch and x.shape[1] == hw.c_in and x.shape[2] >= sp.ny * sp.nx:
             pitch = x.shape[2]                       # (B, c_in, pitch): planes padded by pad_feature
@@ -354,6 +389,7 @@ def head_decode_compact(feats: Sequence[torch.Tensor], weights: Sequence[HeadWei
         for a in range(sp.na):
             s.anchor_vec[a][0], s.anchor_vec[a][1] = av[a][0], av[a][1]
     flags = (_lib.HEAD_ACCUMULATE if accumulate else 0) | (0 if candidates else _lib.HEAD_NO_CANDIDATES)
+    flags |= FEATURE_DTYPE_FLAGS[feats[0].dtype]
     if any(hw.fp32x3 for hw in weights):
         if not all(hw.fp32x3 for hw in weights):
             raise ValueError("fold every head of one call with the same fp32x3 setting")
