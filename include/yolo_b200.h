@@ -47,7 +47,8 @@ typedef struct CUstream_st* yolo_b200_stream_t;
 typedef struct {
     const float* head;      /* (B, na*(5+nc), ny, nx) fp32 NCHW contiguous: the tensor YOLOLayer.forward receives.
                                yolo_b200_decode_compact_ex with YOLO_B200_VARIANT_F16 / _BF16 reads it as fp16 / bf16
-                               elements instead (2-byte aligned; 8-byte aligned planes take 8-byte loads) */
+                               elements instead (2-byte aligned; 8-byte aligned planes take 8-byte loads); with
+                               YOLO_B200_VARIANT_NHWC it is (B, ny, nx, na*(5+nc)) contiguous (channels_last) */
     int32_t ny, nx;         /* grid size (p.shape[-2], p.shape[-1]) */
     int32_t na;             /* anchors of this layer (len(anchors)) */
     int32_t row_off;        /* first row of this scale inside one image of the concatenated prediction
@@ -113,6 +114,13 @@ int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales_host, int n_scales
  * YOLO_B200_E_RANGE, before anything is enqueued.  The other entry points read fp32 only. */
 #define YOLO_B200_VARIANT_F16 0x200
 #define YOLO_B200_VARIANT_BF16 0x400
+/* OR-ed into `variant` of yolo_b200_decode_compact_ex: every scale.head of the call holds the channels_last (NHWC) memory of
+ * its (B, na*(5+nc), ny, nx) tensor, i.e. (B, ny, nx, na*(5+nc)) contiguous -- what a torch.channels_last model hands over.
+ * It is read in place by a kernel that streams those rows of 5+nc logits through a shared-memory ring (one bulk copy per
+ * tile; a head whose base is not 16-byte aligned takes plain loads) and reads every byte.  The candidates are bit-identical
+ * to those of the same call on the NCHW copy of the heads.  Combines with variant 0, _ACCUMULATE, _F16 and _BF16; with
+ * variants 1 to 4 (NCHW kernels) the call returns YOLO_B200_E_UNSUPPORTED before anything is enqueued. */
+#define YOLO_B200_VARIANT_NHWC 0x1000
 
 /* Same candidates, from an already decoded prediction (the tensor model.forward returned):
  * utils.py:210-234.  With write_back_score != 0 the product obj*max_cls is stored into
@@ -162,7 +170,8 @@ int yolo_b200_nms_ex(const yolo_b200_box* cand_box, const yolo_b200_meta* cand_m
  * The caller folds an eval-mode BatchNorm into weight/bias (what ConvBlock.fuse does, models/yolo_base.py:46-57). */
 typedef struct {
     const float* x;          /* (B, c_in, ny, nx) fp32 NCHW contiguous, 16-byte aligned: input of the head convolution.
-                                With YOLO_B200_HEAD_F16 / _BF16: fp16 / bf16 elements, (B, c_in, pitch) */
+                                With YOLO_B200_HEAD_F16 / _BF16: fp16 / bf16 elements, (B, c_in, pitch).  With
+                                YOLO_B200_HEAD_NHWC: (B, ny, nx, c_in) contiguous (channels_last) */
     const float* weight;     /* (256, c_in) fp32 row-major, 16-byte aligned: rows na*(5+nc) .. 255 zero (the kernel's W tile
                                 covers up to 256 output channels; which rows it fetches depends on the instantiation);
                                 (512, c_in) with YOLO_B200_HEAD_FP32X3; (256, c_in) of x's 16-bit type with YOLO_B200_HEAD_F16 /
@@ -200,6 +209,14 @@ typedef struct {
  *   x or weight not 16-byte aligned: YOLO_B200_E_ALIGN. */
 #define YOLO_B200_HEAD_F16           0x10
 #define YOLO_B200_HEAD_BF16          0x20
+/* flags: every x is a channels_last (NHWC) feature map, (B, ny, nx, c_in) contiguous -- what a torch.channels_last model hands
+ * over.  x is then a row-major (B*ny*nx, c_in) matrix: one 3-D tensor-map box per k-block brings 128 positions x 128 bytes of
+ * channels (K-major, SWIZZLE_128B; the ragged last tile of an image is zero-filled), so every plane size (19x19, 13x13, odd
+ * 16-bit planes) is read in place with no loader warps and no padded copy.  Same head values and candidates as the NCHW call.
+ * Combines with YOLO_B200_HEAD_FP32X3, _F16 and _BF16; c_in, anchor and class rules as without it.  Every return code is
+ * decided before anything is enqueued:  x_row_pitch != 0 or _CTA_PAIR: YOLO_B200_E_UNSUPPORTED;  x not 16-byte aligned:
+ * YOLO_B200_E_ALIGN. */
+#define YOLO_B200_HEAD_NHWC          0x40
 #define YOLO_B200_HEAD_PROFILE_MAINLOOP 0x100  /* flags, profiling only (results are garbage): skip the epilogue */
 #define YOLO_B200_HEAD_PROFILE_NO_W     0x200  /* profiling only: the weight tiles are fetched once, not per position tile */
 #define YOLO_B200_HEAD_PROFILE_NO_X     0x400  /* profiling only: the feature tiles are fetched once */
@@ -220,7 +237,8 @@ int yolo_b200_pad_planes_16(const void* x, void* out, long long rows, int plane,
 int yolo_b200_head_supported(int c_in, int ny, int nx, int x_row_pitch, int na, int n_classes);
 /* the same question for a call with `flags` (YOLO_B200_HEAD_FP32X3, YOLO_B200_HEAD_CTA_PAIR: those need a 16-byte row pitch;
  * YOLO_B200_HEAD_F16 / _BF16: c_in % 64 == 0 and an 8-element pitch or even contiguous planes, see yolo_b200_head.x_row_pitch;
- * 0 for both 16-bit bits or for a 16-bit bit with FP32X3 or CTA_PAIR) */
+ * 0 for both 16-bit bits or for a 16-bit bit with FP32X3 or CTA_PAIR; YOLO_B200_HEAD_NHWC: every plane size, x_row_pitch == 0,
+ * not with CTA_PAIR) */
 int yolo_b200_head_supported_ex(int c_in, int ny, int nx, int x_row_pitch, int na, int n_classes, int flags);
 /* Candidates exactly as yolo_b200_decode_compact would produce from the head tensor (same record layout, same count /
  * overflow protocol).  Every wait inside the kernel's pipeline is bounded (10 s of wall-clock time without progress):

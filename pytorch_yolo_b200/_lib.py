@@ -44,12 +44,14 @@ E_UNSUPPORTED = -5
 VARIANT_ACCUMULATE = 0x100
 VARIANT_F16 = 0x200
 VARIANT_BF16 = 0x400
+VARIANT_NHWC = 0x1000
 HEAD_ACCUMULATE = 1
 HEAD_FP32X3 = 8
 HEAD_NO_CANDIDATES = 2
 HEAD_CTA_PAIR = 4
 HEAD_F16 = 0x10
 HEAD_BF16 = 0x20
+HEAD_NHWC = 0x40
 
 
 class YoloB200Error(RuntimeError):

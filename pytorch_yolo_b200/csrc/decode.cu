@@ -6,6 +6,8 @@
 //                              (reference models/yolo_layer.py:57-99 + models/yolov3_spp.py:163-164)
 //   compact_from_dense_kernel  the filter/compaction half of non_max_suppression on an already decoded
 //                              tensor (reference utils/utils.py:210-234), fed by TMA bulk copies
+//   decode_compact_nhwc_kernel decode_compact on channels_last heads: compact_from_dense's bulk-copy ring over the rows of
+//                              5+nc logits, decode_compact's arithmetic
 //
 // All three are HBM-bound streaming kernels that read each input byte at most once.  decode_compact_kernel reads the
 // objectness plane whole and the box and class planes only around positions whose objectness can pass the confidence
@@ -895,6 +897,111 @@ compact_from_dense_kernel(const __grid_constant__ CompactParams P) {
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// decode_compact on channels_last heads (YOLO_B200_VARIANT_NHWC).  The memory of a (B, na*(5+nc), ny, nx) channels_last
+// head is (B, ny, nx, na, 5+nc): B*ny*nx*na rows of 5+nc contiguous logits in (image, y, x, anchor) order -- the layout
+// compact_from_dense streams, so this is its ring: persistent CTAs pull tiles of P.tp rows of one scale into a 2-stage
+// shared-memory ring with one cp.async.bulk each (tail tiles and heads whose base is not 16-byte aligned: a plain copy),
+// and one thread owns one row.  The arithmetic is decode_compact's: the logit-space class scan (skipped where obj_gate
+// shows the objectness cannot pass) and finish_anchor, on values converted to fp32 right after the shared-memory load.
+// Per scale: vec = 4 when the head's base is 16-byte aligned, first_tile = its first tile.
+template <typename T>
+__global__ void __launch_bounds__(kCfThreads)
+decode_compact_nhwc_kernel(const __grid_constant__ DecodeParams P) {
+    extern __shared__ __align__(128) float smem[];
+    __shared__ __align__(8) uint64_t full[kCfStages];
+    const int nc = P.nc, no = nc + 5;
+    const int rows_tile = P.tp;
+    const int tile_elems = rows_tile * no;
+    T* ring = reinterpret_cast<T*>(smem);
+    const int tid = threadIdx.x;
+
+    if (tid == 0) {
+#pragma unroll
+        for (int s = 0; s < kCfStages; ++s) mbar_init(&full[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+
+    // tile -> (scale, first row of the scale's B*plane*na rows, rows in the tile)
+    auto locate = [&](int t, int& sc, long long& r0, int& rows) {
+        sc = 0;
+#pragma unroll
+        for (int k = 1; k < YOLO_B200_MAX_SCALES; ++k)
+            if (k < P.n_scales && t >= P.sc[k].first_tile) sc = k;
+        const ScaleDev& S = P.sc[sc];
+        r0 = (long long)(t - S.first_tile) * rows_tile;
+        rows = (int)min((long long)rows_tile, (long long)P.batch * S.na * S.plane - r0);
+    };
+    auto tile_is_tma = [&](int sc, int rows) -> bool { return P.sc[sc].vec == 4 && rows == rows_tile; };
+    auto issue = [&](int t, int stage) {
+        int sc, rows;
+        long long r0;
+        locate(t, sc, r0, rows);
+        if (tile_is_tma(sc, rows)) {
+            const uint32_t bytes = (uint32_t)tile_elems * (uint32_t)sizeof(T);
+            fence_proxy_async_smem();                  // earlier generic-proxy accesses of the stage before the bulk copy
+            mbar_expect_tx(&full[stage], bytes);
+            tma_bulk_g2s(ring + (size_t)stage * tile_elems, static_cast<const T*>(P.sc[sc].head) + r0 * no, bytes, &full[stage]);
+        }
+    };
+
+    uint32_t phase_bits = 0;
+    int t = blockIdx.x;
+    if (tid == 0) {
+        int tt = t;
+#pragma unroll
+        for (int s = 0; s < kCfStages; ++s, tt += gridDim.x)
+            if (tt < P.n_tiles) issue(tt, s);
+    }
+    for (int it = 0; t < P.n_tiles; t += gridDim.x, ++it) {
+        const int stage = it % kCfStages;
+        T* tl = ring + (size_t)stage * tile_elems;
+        int sc, rows;
+        long long r0;
+        locate(t, sc, r0, rows);
+        const ScaleDev& S = P.sc[sc];
+        if (tile_is_tma(sc, rows)) {
+            mbar_wait(&full[stage], (phase_bits >> stage) & 1u);
+            phase_bits ^= 1u << stage;
+        } else {
+            const T* src = static_cast<const T*>(S.head) + r0 * no;
+            for (int i = tid; i < rows * no; i += kCfThreads) tl[i] = src[i];
+            __syncthreads();
+        }
+
+        // row g = ((img * ny + y) * nx + x) * na + a of the scale: anchor row row_off + a * plane + y * nx + x
+        const bool active = tid < rows;
+        const long long g = r0 + (active ? tid : 0);
+        const int q = (int)(g / S.na);
+        const int a = (int)(g - (long long)q * S.na);
+        const int img = q / S.plane;
+        const int pos = q - img * S.plane;
+        const T* r = tl + (active ? tid : 0) * no;
+        const float t4 = to_f32(r[4]);
+        const bool gate = active && obj_gate(t4, P.conf);
+        float t0 = 0.0f, t1 = 0.0f, t2 = 0.0f, t3 = 0.0f;
+        float m = __int_as_float(0xff800000), m2 = m;
+        int idx = 0;
+        if (gate) {                                   // finish_anchor reads none of these for a gated-off row
+            t0 = to_f32(r[0]); t1 = to_f32(r[1]); t2 = to_f32(r[2]); t3 = to_f32(r[3]);
+            if (nc > 1) {
+                for (int c = 0; c < nc; ++c) {
+                    const float x = to_f32(r[5 + c]);
+                    const bool up = x > m;
+                    m2 = up ? m : fmaxf(m2, x);
+                    idx = up ? c : idx;
+                    m = fmax_nan(m, x);
+                }
+            }
+        }
+        finish_anchor(P, S, gate, img, a, pos, t0, t1, t2, t3, t4, m, m2, idx, r + 5, 1);
+        __syncthreads();                       // everyone is done with this stage
+        const int nt = t + kCfStages * gridDim.x;
+        if (tid == 0 && nt < P.n_tiles) issue(nt, stage);
+    }
+}
+
 }  // namespace yb
 
 // ================================================================================================
@@ -1024,19 +1131,57 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     if (!cand_box || !cand_meta || !count || !overflow) return YOLO_B200_E_NULL;
     const bool accumulate = variant >= 0 && (variant & YOLO_B200_VARIANT_ACCUMULATE) != 0;
     if (accumulate) variant &= ~YOLO_B200_VARIANT_ACCUMULATE;
+    const bool nhwc = variant >= 0 && (variant & YOLO_B200_VARIANT_NHWC) != 0;
+    if (nhwc) variant &= ~YOLO_B200_VARIANT_NHWC;
     const int half_bits = variant >= 0 ? variant & (YOLO_B200_VARIANT_F16 | YOLO_B200_VARIANT_BF16) : 0;
     variant &= ~half_bits;
     if (cap_per_img < 1 || variant < 0 || variant > 4) return YOLO_B200_E_RANGE;
     if (half_bits == (YOLO_B200_VARIANT_F16 | YOLO_B200_VARIANT_BF16)) return YOLO_B200_E_RANGE;
     if (half_bits && (variant == 2 || variant == 3)) return YOLO_B200_E_UNSUPPORTED;     // the TMA kernels read fp32 only
+    if (nhwc && variant != 0) return YOLO_B200_E_UNSUPPORTED;                          // variants 1-4 are NCHW kernels
     if ((((uintptr_t)cand_box) | ((uintptr_t)cand_meta)) & 15u) return YOLO_B200_E_ALIGN;
     const bool gated = variant <= 1;
     DecodeParams P{};
-    const int blocks = fill_params(P, scales, n_scales, batch, nc, rows_per_img, false, accumulate, half_bits ? 2 : 4);
+    const int esize = half_bits ? 2 : 4;
+    const int blocks = fill_params(P, scales, n_scales, batch, nc, rows_per_img, false, accumulate, esize);
     if (blocks < 0) return blocks;
     P.conf = conf_thres; P.min_wh = min_wh;
     P.cand_box = cand_box; P.cand_meta = cand_meta; P.cap = cap_per_img; P.count = count; P.overflow = overflow;
     const int no = nc + 5;
+    cudaError_t e;
+    if (nhwc) {
+        // rows per tile as compact_from_dense picks them: as many as fit a 2-stage ring (128 for 85 columns), halved down
+        // to 4 fp32 / 8 16-bit rows at most, which keeps every tile a multiple of 16 bytes for odd 5+nc
+        const int min_rows = 16 / esize;
+        int rows_tile = kCfRows;
+        while (rows_tile > min_rows && (size_t)kCfStages * rows_tile * no * esize > 200 * 1024) rows_tile >>= 1;
+        const size_t smem = (size_t)kCfStages * rows_tile * no * esize;
+        if (smem > 200 * 1024) return YOLO_B200_E_RANGE;
+        long long tiles = 0;
+        for (int k = 0; k < n_scales; ++k) {
+            ScaleDev& d = P.sc[k];
+            d.first_tile = (int)tiles;
+            d.vec = ((uintptr_t)d.head & 15u) == 0 ? 4 : 1;          // bulk copies need a 16-byte aligned base
+            tiles += ((long long)batch * d.na * d.plane + rows_tile - 1) / rows_tile;
+        }
+        for (int k = n_scales; k < YOLO_B200_MAX_SCALES; ++k) P.sc[k].first_tile = 0x7fffffff;
+        if (tiles > 0x7fffffffLL) return YOLO_B200_E_RANGE;
+        P.tp = rows_tile;
+        P.n_tiles = (int)tiles;
+        const void* kern = half_bits == YOLO_B200_VARIANT_F16    ? (const void*)decode_compact_nhwc_kernel<__half>
+                         : half_bits == YOLO_B200_VARIANT_BF16   ? (const void*)decode_compact_nhwc_kernel<__nv_bfloat16>
+                                                                 : (const void*)decode_compact_nhwc_kernel<float>;
+        if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return (int)e;
+        if (!accumulate && (e = zero_counters(count, overflow, batch, stream)) != cudaSuccess) return (int)e;
+        if (blocks == 0) return 0;
+        int dev = 0, sms = 148;
+        if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        const int per_sm = (int)((220 * 1024) / (smem + 1024));
+        const int grid = (int)min((long long)sms * (per_sm < 1 ? 1 : per_sm), tiles);
+        void* args[] = {&P};
+        if ((e = cudaLaunchKernel(kern, dim3(grid), dim3(kCfThreads), args, smem, stream)) != cudaSuccess) return (int)e;
+        return (int)cudaGetLastError();
+    }
     const int tp = tma_tile_positions(no);
     // Measured on B200 (profiles/r01_c_decode_variants.txt): the dense LDG kernel streams at 5.8 TB/s, the 1-D bulk-copy
     // ring at 3.1 TB/s (one cp.async.bulk per 1 KB channel row: TMA issue-bound), so "automatic" means LDG, and the gated
@@ -1046,7 +1191,6 @@ extern "C" int yolo_b200_decode_compact_ex(const yolo_b200_scale* scales, int n_
     // refusals come before the counters are zeroed: a refused call must leave the counts of an earlier call intact
     if (use_tma && tp == 0) return YOLO_B200_E_RANGE;
     if (variant == 3 && no > 256) return YOLO_B200_E_RANGE;            // a TMA box is at most 256 rows
-    cudaError_t e;
     if (!accumulate && (e = zero_counters(count, overflow, batch, stream)) != cudaSuccess) return (int)e;
     if (blocks == 0) return 0;
 

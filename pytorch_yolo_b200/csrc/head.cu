@@ -34,6 +34,12 @@
 // A stage is 16 KB of X + NPAD x 128 bytes of W: the same 48 KB as the fp32 stage.  Planes without a 16-byte pitch
 // (plane % 8 != 0) but with 4-byte aligned rows (even planes) are filled by the loader warps with 8-byte (plane % 4 == 0)
 // or 4-byte copies; odd planes are padded by the host first (yolo_b200_pad_planes_16).
+//
+// channels_last feature maps (YOLO_B200_HEAD_NHWC, HeadParams.nhwc, uniform per launch): X is a row-major
+// (B*plane, c_in) matrix, so A is K-major like W.  One 3-D box of (c_in, plane, batch) per k-block -- BK channels (128
+// bytes) x 128 positions x 1 image, SWIZZLE_128B, positions past the plane zero-filled -- and the A descriptor of B
+// (SBO 1 KB, +32 bytes per MMA K step) with the instruction descriptor's A-major bit clear.  Every plane size is read in
+// place (no loader warps, no padded copy); the W ring, the epilogue and head_out are unchanged.
 #include <cuda.h>          // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 
 #include "common.cuh"
@@ -90,6 +96,8 @@ struct HeadParams {
     int32_t* count;
     int32_t* overflow;
     int emit;                              // 0: only write head_out (convolution only)
+    int nhwc;                              // channels_last X (YOLO_B200_HEAD_NHWC): tmap_x is the 3-D (c_in, plane, batch)
+                                           // map, one box per k-block, and A is K-major (read by the producer and the MMA thread)
     int skip_epilogue;                     // profiling bits (8 = the MMA thread only recycles the stages): 1 = epilogue warps only release the accumulator, 2 = W fetched
                                            // only for the first ring round, 4 = X fetched only for the first ring round
 };
@@ -206,6 +214,8 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo_bytes,
     d |= (uint64_t)layout << 61;
     return d;
 }
+// the descriptor `fixed` (built with address 0) pointed at addr
+__device__ __forceinline__ uint64_t smem_desc_at(uint64_t fixed, uint32_t addr) { return fixed | (uint64_t)((addr >> 4) & 0x3fffu); }
 // Instruction descriptor: fp32 accumulator, tf32 A and B, A MN-major (positions contiguous), B K-major, M x N tile.
 __host__ __device__ constexpr uint32_t instr_desc_tf32(int m, int n) {
     return (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (0u << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
@@ -546,10 +556,12 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                     // profiling modes (bits 1, 2 of skip_epilogue): fetch W / X only during the first trip round the ring
                     const bool load_w = !(P.skip_epilogue & 2) || it < (uint32_t)kStages;
                     const bool load_x = (!(P.skip_epilogue & 4) || it < (uint32_t)kStages) && !S.manual;   // manual: the loader warps
-                    mbar_expect_tx(&full[st], (uint32_t)((load_x ? (one_box ? kABytes : atoms * kAtom) : 0) +
+                    mbar_expect_tx(&full[st], (uint32_t)((load_x ? (one_box || P.nhwc ? kABytes : atoms * kAtom) : 0) +
                                                          (load_w ? (X3 ? 2 : 1) * kBBytes : 0)));
                     if (load_x) {
-                        if (one_box)
+                        if (P.nhwc)       // [BK channels = 128 bytes] x [128 positions] of one image; rows past the plane zero
+                            tma_tile3_g2s(a_s, &S.tmap_x, kb * BK, p0, img, &full[st]);
+                        else if (one_box)
                             tma_tile3_g2s(a_s, &S.tmap_x3, 0, img * S.c_in + kb * BK, p0 >> AS, &full[st]);
                         else
                             for (int j = 0; j < atoms; ++j)
@@ -568,7 +580,14 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
     } else if (warp == 1) {
         // ===== MMA issuer =====
         if (lane == 0) {
-            constexpr uint32_t idesc = H ? instr_desc_f16(kM, NPAD, DT == kDtBF16) : instr_desc_tf32(kM, NPAD);
+            constexpr uint32_t idesc_mn = H ? instr_desc_f16(kM, NPAD, DT == kDtBF16) : instr_desc_tf32(kM, NPAD);
+            // channels_last X: A is K-major (bit 15 clear) in the SWIZZLE_128B layout of B -- 8-position groups 1 KB apart
+            // (SBO), each MMA's K step 32 bytes further along the 128-byte row (8 tf32 or 16 16-bit channels)
+            const bool nhwc = P.nhwc != 0;
+            const uint32_t idesc = nhwc ? idesc_mn & ~(1u << 15) : idesc_mn;
+            const uint32_t a_step = nhwc ? 32u : (H ? 2048u : 1024u);
+            const uint64_t a_fixed = nhwc ? smem_desc(0, 16u, 1024u, kSw128)
+                                          : H ? smem_desc(0, kAtomBytes16, 1024u, kSw128) : smem_desc(0, kAtomBytes, 512u, kSw128Base32);
             uint32_t it = 0, xparity = 0;
             int tl = 0;
             for (int tile = blockIdx.x; tile < P.n_tiles; tile += gridDim.x, ++tl) {
@@ -599,7 +618,7 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                             //    the tile's two 64-position atoms are kAtomBytes16 apart (LBO), 8-channel groups 1 KB apart
                             //    (SBO), so this instruction's 16 channels start 2 KB after the previous one's
                             // B: K-major, as in fp32: 8-row groups 1 KB apart (SBO); 16 channels = 32 bytes inside the row
-                            const uint64_t ad = smem_desc(a_s + (uint32_t)kk * 2048u, kAtomBytes16, 1024u, kSw128);
+                            const uint64_t ad = smem_desc_at(a_fixed, a_s + (uint32_t)kk * a_step);
                             const uint64_t bd = smem_desc(b_s + (uint32_t)kk * 32u, 16u, 1024u, kSw128);
                             umma_f16(d_tmem, ad, bd, idesc, (kb | kk) != 0);
                         }
@@ -610,11 +629,11 @@ head_decode_compact_kernel(const __grid_constant__ HeadParams P) {
                         //    128-byte row, a swizzle atom is 4 rows, so this instruction's 8 channels are two atoms 512 bytes
                         //    apart (SBO) and the next instruction starts 1 KB further
                         // B: K-major, 8-row groups 1 KB apart (SBO); 8 channels = 32 bytes inside the 128-byte row
-                        const uint64_t ad = smem_desc(a_s + (uint32_t)kk * 1024u, kAtomBytes, 512u, kSw128Base32);
+                        const uint64_t ad = smem_desc_at(a_fixed, a_s + (uint32_t)kk * a_step);
                         const uint64_t bd = smem_desc(b_s + (uint32_t)kk * 32u, 16u, 1024u, kSw128);
                         umma_tf32(d_tmem, ad, bd, idesc, (kb | kk) != 0);
                         if constexpr (X3) {
-                            const uint64_t ad_lo = smem_desc(a_s + kABytes + (uint32_t)kk * 1024u, kAtomBytes, 512u, kSw128Base32);
+                            const uint64_t ad_lo = smem_desc_at(a_fixed, a_s + kABytes + (uint32_t)kk * a_step);
                             const uint64_t bd_lo = smem_desc(b_s + kBBytes + (uint32_t)kk * 32u, 16u, 1024u, kSw128);
                             umma_tf32(d_tmem, ad, bd_lo, idesc, true);
                             umma_tf32(d_tmem, ad_lo, bd, idesc, true);
@@ -1134,6 +1153,14 @@ static int head_dtype(int flags) {
 
 extern "C" int yolo_b200_head_supported_ex(int c_in, int ny, int nx, int x_row_pitch, int na, int n_classes, int flags) {
     const int dt = head_dtype(flags);
+    if (flags & YOLO_B200_HEAD_NHWC) {
+        // channels_last X: one tensor-map box per k-block whatever the plane, no row pitch; not the CTA-pair kernel
+        if (dt < 0 || x_row_pitch != 0 || (flags & YOLO_B200_HEAD_CTA_PAIR)) return 0;
+        if (dt != hd::kDtF32 && (flags & YOLO_B200_HEAD_FP32X3)) return 0;
+        const int bk = dt != hd::kDtF32 ? hd::kBK16 : hd::kBK;
+        if (c_in < bk || c_in % bk != 0 || ny < 1 || nx < 1) return 0;
+        return head_kernel_for(na, n_classes, false, false, false, false, dt) != nullptr ? 1 : 0;
+    }
     if (dt != hd::kDtF32) {
         // 16-bit: one-pass single-CTA kernel, 64-channel k-blocks, a row pitch of 8 elements (16 bytes) unless the
         // contiguous planes are even (the loader warps copy 4-byte aligned pieces; odd planes go through the padded copy)
@@ -1171,6 +1198,8 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
     if (dt < 0) return YOLO_B200_E_RANGE;
     const bool h16 = dt != hd::kDtF32;
     if (h16 && (flags & (YOLO_B200_HEAD_FP32X3 | YOLO_B200_HEAD_CTA_PAIR))) return YOLO_B200_E_UNSUPPORTED;
+    const bool nhwc = (flags & YOLO_B200_HEAD_NHWC) != 0;
+    if (nhwc && (flags & YOLO_B200_HEAD_CTA_PAIR)) return YOLO_B200_E_UNSUPPORTED;
     if (emit && (!cand_box || !cand_meta)) return YOLO_B200_E_NULL;
     if (n_heads < 1 || n_heads > YOLO_B200_MAX_SCALES || batch < 0 || nc < 1 || rows_per_img < 1 || (emit && cap_per_img < 1))
         return YOLO_B200_E_RANGE;
@@ -1239,9 +1268,19 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
             const int plane = h.scale.ny * h.scale.nx;
             const uint64_t pitch = h.x_row_pitch ? (uint64_t)h.x_row_pitch : (uint64_t)plane;      // elements between channel planes
             int rc;
-            S.manual = pitch % (16 / esz) != 0 ? 1 : 0;   // (validated above: contiguous planes, one-pass single-CTA kernel)
+            S.manual = !nhwc && pitch % (16 / esz) != 0 ? 1 : 0;   // (validated above: contiguous planes, one-pass single-CTA kernel)
             S.x = h.x;
-            if (!S.manual &&
+            if (nhwc) {
+                // channels_last: (c_in, plane, batch), box = one k-block of channels (128 bytes) x 128 positions x 1 image,
+                // positions past the plane zero-filled; c_in * esz is a multiple of 128 bytes
+                const cuuint64_t gdim[3] = {(cuuint64_t)h.c_in, (cuuint64_t)plane, (cuuint64_t)batch};
+                const cuuint64_t gstride[2] = {(cuuint64_t)h.c_in * esz, (cuuint64_t)plane * h.c_in * esz};
+                const cuuint32_t box[3] = {(cuuint32_t)bk, (cuuint32_t)hd::kM, 1};
+                const cuuint32_t estr[3] = {1, 1, 1};
+                if (encode(&S.tmap_x, x_type, 3, const_cast<float*>(h.x), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                           CU_TENSOR_MAP_SWIZZLE_128B, x_promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+                    return YOLO_B200_E_RANGE;
+            } else if (!S.manual &&
                 (rc = encode_2d(encode, &S.tmap_x, h.x, (uint64_t)plane, (uint64_t)batch * h.c_in, pitch * esz, ap, bk, x_swizzle, x_promo, x_type)))
                 return rc;
             // (three-pass mode: the tensor holds 512 rows, the low parts of the weights behind the weights)
@@ -1254,7 +1293,7 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
             // 3-D view over the complete atoms (32 positions, 16-bit: 64) of every row; rows are pitch elements apart, atoms
             // 128 bytes; the box is the tile's four (16-bit: two) atoms
             S.use_x3 = 0;
-            if (plane >= ap && !S.manual) {
+            if (!nhwc && plane >= ap && !S.manual) {
                 const cuuint64_t gdim[3] = {(cuuint64_t)ap, (cuuint64_t)batch * h.c_in, (cuuint64_t)(plane / ap)};
                 const cuuint64_t gstride[2] = {(cuuint64_t)pitch * esz, 128};
                 const cuuint32_t box[3] = {(cuuint32_t)ap, (cuuint32_t)bk, (cuuint32_t)(hd::kM / ap)};
@@ -1279,6 +1318,7 @@ extern "C" int yolo_b200_head_decode_compact(const yolo_b200_head* heads, int n_
         P.conf = conf_thres; P.min_wh = min_wh;
         P.cand_box = cand_box; P.cand_meta = cand_meta; P.cap = cap_per_img; P.count = count; P.overflow = overflow;
         P.emit = emit ? 1 : 0;
+        P.nhwc = nhwc ? 1 : 0;
         P.skip_epilogue = (flags >> 8) & 15;     // YOLO_B200_HEAD_PROFILE_* bits
 
         // The CTA-pair kernel is exact but measured ~5 % slower than the single-CTA kernel on B200 (profiles/r01_m_*): on

@@ -119,14 +119,15 @@ class Detector:
         with torch.cuda.graph(g):          # the side stream forks from / joins torch's capture stream: one graph, two priorities
             self._enqueue(inputs)
         self._graph = g
-        self._bound = (tuple((h.data_ptr(), h.dtype) for h in inputs), inputs)
+        self._bound = (tuple((h.data_ptr(), h.dtype, h.stride()) for h in inputs), inputs)
 
     def launch(self, inputs: Sequence[torch.Tensor]) -> None:
         """Enqueue one step on the current stream (no host sync)."""
         self._stream = torch.cuda.current_stream(self.device)
         if self.use_graph:
-            # the dtype picks the kernel: a 16-bit tensor at a freed fp32 tensor's address needs a new graph
-            ptrs = tuple((h.data_ptr(), h.dtype) for h in inputs)
+            # the dtype and the layout pick the kernel: a 16-bit tensor at a freed fp32 tensor's address, or a channels_last
+            # tensor at an NCHW tensor's address (or the reverse), needs a new graph
+            ptrs = tuple((h.data_ptr(), h.dtype, h.stride()) for h in inputs)
             if self._bound is None or self._bound[0] != ptrs:
                 self.bind(inputs)
             self._graph.replay()
@@ -237,7 +238,8 @@ class PipelinedDetector:
         ticket = self._next
         lane = ticket % self.depth
         if self._staging[lane] is None:
-            self._staging[lane] = [torch.empty(h.shape, dtype=h.dtype, device=self.device) for h in host_inputs]
+            # empty_like keeps the layout: a channels_last batch stays channels_last (a plain copy, then the NHWC kernel)
+            self._staging[lane] = [torch.empty_like(h, device=self.device) for h in host_inputs]
         stage = self._staging[lane]
         with torch.cuda.stream(self.streams[lane]):
             for d, h in zip(stage, host_inputs):

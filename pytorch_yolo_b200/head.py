@@ -24,6 +24,10 @@ fp16 / bf16 feature maps (``feature_dtype``, what a ``.half()`` model or autocas
 ``kind::f16`` main loop: exact products of the 16-bit operands (the weights are folded in fp64 and rounded to that type),
 fp32 accumulation, and the same fp32 epilogue.  Such scales need c_in % 64 == 0; odd planes (19x19, 13x13) go through
 the 16-bit padded copy; uncovered scales run the module's own convolution under ``torch.autocast`` of that type.
+
+channels_last feature maps (a ``torch.channels_last`` model) are read in place by the same kernel with a K-major A operand,
+at every plane size: no padded copy.  The unfused scales' module outputs are then channels_last too, and
+``decode_compact`` reads them in place.
 """
 from __future__ import annotations
 
@@ -117,7 +121,9 @@ class HeadDetector(Detector):
                                 f"feature_dtype={self.feature_dtype}")
         first = True
         if any(self.fused):
-            feats = [x if p is None else ops.pad_feature(x, out=p) for x, p in zip(feats, self.padded)]
+            # channels_last maps are read in place at every plane size (one NHWC call, no padded copy)
+            if not all(ops.is_channels_last(x) for x in self._pick(feats, True)):
+                feats = [x if p is None else ops.pad_feature(x, out=p) for x, p in zip(feats, self.padded)]
             ops.head_decode_compact(self._pick(feats, True), self._pick(self.weights, True), self._pick(self.specs, True),
                                     self._pick(self.row_offs, True), self.rows, self.nc, self.conf_thres, self.buf)
             first = False

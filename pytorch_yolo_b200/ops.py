@@ -44,6 +44,13 @@ def _require_dtype(t: torch.Tensor, what: str, dtypes) -> None:
         raise TypeError(f"{what}: expected {' or '.join(str(d).replace('torch.', '') for d in dtypes)}, got {t.dtype}")
 
 
+def is_channels_last(t: torch.Tensor) -> bool:
+    """Is the memory of this 4-D tensor channels_last and not also NCHW contiguous?  Such tensors (what a
+    ``torch.channels_last`` model hands over) are read in place by the NHWC kernels.  A tensor that is both (1x1 grids,
+    one channel) is NCHW to every kernel; any other layout is copied to NCHW first."""
+    return t.dim() == 4 and t.is_contiguous(memory_format=torch.channels_last) and not t.is_contiguous()
+
+
 def _stream_ptr(device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
 
@@ -74,7 +81,7 @@ def scale_spec(anchors, ny: int, nx: int, img_size) -> ScaleSpec:
     return ScaleSpec(tuple((float(a), float(b)) for a, b in anchors), int(ny), int(nx), float(stride), vec)
 
 
-def _fill_scales(heads: Sequence[torch.Tensor], specs: Sequence[ScaleSpec], nc: int, dtypes=_FP32):
+def _fill_scales(heads: Sequence[torch.Tensor], specs: Sequence[ScaleSpec], nc: int, dtypes=_FP32, nhwc: bool = False):
     if not 1 <= len(heads) <= MAX_SCALES or len(heads) != len(specs):
         raise ValueError(f"need 1..{MAX_SCALES} heads with one spec each, got {len(heads)} / {len(specs)}")
     arr = (Scale * len(heads))()
@@ -91,7 +98,7 @@ def _fill_scales(heads: Sequence[torch.Tensor], specs: Sequence[ScaleSpec], nc: 
             raise ValueError(f"all heads of one call must share a dtype: head 0 is {heads[0].dtype}, head {k} {h.dtype}")
         if h.dim() != 4 or h.shape[1] != sp.na * (nc + 5) or h.shape[2] != sp.ny or h.shape[3] != sp.nx:
             raise ValueError(f"head {k}: expected (B, {sp.na * (nc + 5)}, {sp.ny}, {sp.nx}), got {tuple(h.shape)}")
-        if not h.is_contiguous():
+        if not nhwc and not h.is_contiguous():
             h = h.contiguous()          # the reference's .view at yolo_layer.py:67 needs contiguity as well
         keep.append(h)
         s = arr[k]
@@ -197,10 +204,13 @@ def decode_compact(heads, specs, nc: int, conf_thres: float, buf: Buffers, min_w
     them, so the candidates are bit-identical to those of ``[h.float() for h in heads]``; the TMA variants read float32
     only.
     ``variant``: "auto" | "ldg" | "tma" | "tma2d" | "ldg_dense" (identical results; see include/yolo_b200.h).
+    With "auto" and every head channels_last (:func:`is_channels_last`) the heads are read in place by the NHWC kernel,
+    with the same candidates as on their NCHW copies; otherwise channels_last heads are copied to NCHW first.
     ``row_offs`` / ``rows_per_img`` / ``accumulate``: decode only some scales of a model and append to the candidates
     already in ``buf`` (the other scales went through :func:`head_decode_compact`)."""
     lib = _lib.load()
-    arr, keep, batch, rows, dev = _fill_scales(heads, specs, nc, tuple(HEAD_DTYPE_BITS))
+    nhwc = variant == "auto" and all(isinstance(h, torch.Tensor) and is_channels_last(h) for h in heads)
+    arr, keep, batch, rows, dev = _fill_scales(heads, specs, nc, tuple(HEAD_DTYPE_BITS), nhwc=nhwc)
     if row_offs is not None:
         for k, off in enumerate(row_offs):
             arr[k].row_off = int(off)
@@ -212,7 +222,7 @@ def decode_compact(heads, specs, nc: int, conf_thres: float, buf: Buffers, min_w
                                               buf.cand_box.data_ptr(), buf.cand_meta.data_ptr(), buf.cap,
                                               buf.count_ptr, buf.overflow_ptr,
                                               DECODE_VARIANTS[variant] | (_lib.VARIANT_ACCUMULATE if accumulate else 0)
-                                              | HEAD_DTYPE_BITS[keep[0].dtype],
+                                              | HEAD_DTYPE_BITS[keep[0].dtype] | (_lib.VARIANT_NHWC if nhwc else 0),
                                               _stream_ptr(dev)),
               "yolo_b200_decode_compact")
 
@@ -298,12 +308,16 @@ def fold_head(module: torch.nn.Module, device=None, fp32x3: bool = False, dtype:
 
 
 def head_supported(c_in: int, spec: ScaleSpec, nc: int, row_pitch: int = 0, fp32x3: bool = False,
-                   dtype: torch.dtype = torch.float32) -> bool:
+                   dtype: torch.dtype = torch.float32, memory_format: torch.memory_format = torch.contiguous_format) -> bool:
     """Does the tensor-core kernel take this scale?  Contiguous planes that are not a multiple of 4 floats (19x19, 13x13) are
     read in place by the one-pass kernel; the three-pass mode needs them padded (``row_pitch = padded_pitch(spec)``).
     ``dtype`` float16 / bfloat16: feature maps of that type (c_in a multiple of 64; planes that are not a multiple of 8
-    elements are read in place when even, odd ones need ``row_pitch = padded_pitch(spec, dtype)``)."""
+    elements are read in place when even, odd ones need ``row_pitch = padded_pitch(spec, dtype)``).
+    ``memory_format=torch.channels_last``: channels_last feature maps, read in place at every plane size (no row pitch)."""
+    if memory_format not in (torch.contiguous_format, torch.channels_last):
+        raise ValueError(f"memory_format is torch.contiguous_format or torch.channels_last, got {memory_format}")
     flags = (_lib.HEAD_FP32X3 if fp32x3 else 0) | FEATURE_DTYPE_FLAGS[dtype]
+    flags |= _lib.HEAD_NHWC if memory_format == torch.channels_last else 0
     return bool(_lib.load().yolo_b200_head_supported_ex(c_in, spec.ny, spec.nx, row_pitch, spec.na, nc, flags))
 
 
@@ -344,11 +358,14 @@ def head_decode_compact(feats: Sequence[torch.Tensor], weights: Sequence[HeadWei
     accumulator into ``buf``.  ``feats[k]``: (B, c_in, ny, nx) input of head k; ``row_offs[k]``: first row of scale k in the
     concatenated prediction.  The feature maps are float32, float16 or bfloat16, one dtype for all and the one the weights
     were folded to (``fold_head(..., dtype=)``).  ``head_outs[k]`` (optional) receives the activated head tensor (B, na*(5+nc), ny, nx).
-    ``cta_pair`` selects the tcgen05 ``cta_group::2`` variant of the kernel (identical results)."""
+    ``cta_pair`` selects the tcgen05 ``cta_group::2`` variant of the kernel (identical results).
+    When every feature map is channels_last (:func:`is_channels_last`) and ``cta_pair`` is off, the maps are read in place
+    (any plane size, no padded copy); otherwise channels_last maps are copied to NCHW first."""
     lib = _lib.load()
     n = len(feats)
     if not 1 <= n <= MAX_SCALES or not (len(weights) == len(specs) == len(row_offs) == n):
         raise ValueError("one weight set, spec and row offset per head is required")
+    nhwc = not cta_pair and all(isinstance(x, torch.Tensor) and is_channels_last(x) for x in feats)
     arr = (_lib.Head * n)()
     keep = []
     dev = feats[0].device
@@ -372,7 +389,7 @@ def head_decode_compact(feats: Sequence[torch.Tensor], weights: Sequence[HeadWei
             raise ValueError(f"head {k}: {hw.n_out} output channels, expected {sp.na * (nc + 5)}")
         if hw.weight.device != dev:
             raise ValueError("weights must live on the feature maps' device")
-        x = x if x.is_contiguous() else x.contiguous()
+        x = x if nhwc or x.is_contiguous() else x.contiguous()
         bias_c = hw.bias_array()
         keep += [x, bias_c]
         h = arr[k]
@@ -389,7 +406,7 @@ def head_decode_compact(feats: Sequence[torch.Tensor], weights: Sequence[HeadWei
         for a in range(sp.na):
             s.anchor_vec[a][0], s.anchor_vec[a][1] = av[a][0], av[a][1]
     flags = (_lib.HEAD_ACCUMULATE if accumulate else 0) | (0 if candidates else _lib.HEAD_NO_CANDIDATES)
-    flags |= FEATURE_DTYPE_FLAGS[feats[0].dtype]
+    flags |= FEATURE_DTYPE_FLAGS[feats[0].dtype] | (_lib.HEAD_NHWC if nhwc else 0)
     if any(hw.fp32x3 for hw in weights):
         if not all(hw.fp32x3 for hw in weights):
             raise ValueError("fold every head of one call with the same fp32x3 setting")
